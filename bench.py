@@ -73,7 +73,13 @@ def parse(argv=None):
     ap.add_argument("--ref-seconds", type=float, default=150.0, help="budget of the --impl reference run")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary records (tracking workload, icp_mode 3, e2e_cloud, loop closure, kernel mode, sharded)")
     ap.add_argument("--no-speculate", action="store_true", help="LIMU_OPT_SPECULATE off (A/B)")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed windows of `value`, write what their last timed step returned "
+                    "(rank 0) as DIR/pose.npy and DIR/frame_stats.npy (float64), to compare two builds on the same seeded inputs; "
+                    "needs --impl b200 and --steps >= 1")
+    args = ap.parse_args(argv)
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs writes the last timed step of the b200 path: it needs --impl b200 and --steps >= 1")
+    return args
 
 
 def dist_env():
@@ -311,6 +317,18 @@ def parity_record(args, scans, gpu_poses, gpu_frames, cpu):
             "n_keypoints_equal": bool([int(f[0]) for f in gpu_frames[:n]] == [s[1] for s in cpu["sizes"][:n]]),
             "tolerance": "1e-5 m / 1e-6 (quaternion components) per update (north star)", "ok": bool(dp[:, 4:].max() < 1e-5 and dp[:, :4].max() < 1e-6 and g_it == its),
             "against": f"oracle/_ref ({cpu['kind']}: the reference's own sources compiled) for poses and cloud sizes; oracle C port for iterations"}
+
+
+FRAME_STATS_ORDER = ("n_points", "n_down", "n_keypoints", "sigma", "icp.iterations", "icp.converged", "icp.last_ncorr", "icp.mean_candidates",
+                     "icp.miss_fraction", "deskewed")
+
+
+def dump_outputs(out_dir, pose, stats):
+    """What one register_frame_dev call hands its caller: the pose {qx,qy,qz,qw,tx,ty,tz} and the FrameStats it fills, as FRAME_STATS_ORDER."""
+    os.makedirs(out_dir, exist_ok=True)
+    row = [getattr(stats.icp, k[4:]) if k.startswith("icp.") else getattr(stats, k) for k in FRAME_STATS_ORDER]
+    np.save(os.path.join(out_dir, "pose.npy"), np.asarray(pose, np.float64))
+    np.save(os.path.join(out_dir, "frame_stats.npy"), np.asarray(row, np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------------------------ GPU side
@@ -673,7 +691,7 @@ def main():
     # -- arm 2: inputs resident in HBM (the `value`)
     frames = []
 
-    def dev_step_factory(devs, rec=None):
+    def dev_step_factory(devs, rec=None, returned=None):
         def mk():
             if rec is not None:
                 rec.clear()
@@ -681,7 +699,9 @@ def main():
             def step(o, i, last):
                 if not last and i + 1 < len(devs):
                     o.hint_next_dev(devs[i + 1].data_ptr(), n_pts)   # replay hint (LIMU_OPT_SPECULATE): never across the warm-up / timed boundary
-                o.register_frame_dev(devs[i].data_ptr(), n_pts)
+                pose = o.register_frame_dev(devs[i].data_ptr(), n_pts)
+                if returned is not None:
+                    returned["pose"] = pose
                 if rec is not None:
                     st = o.stats
                     rec.append((st.n_keypoints, st.icp.iterations, st.icp.mean_candidates, st.icp.miss_fraction, st.n_down))
@@ -690,8 +710,11 @@ def main():
 
     flush.fill_(2)
     launches0 = pkg.kernel_launches()
-    val, odom = b.run_windows(dev_step_factory(dev_scans, frames), W, K, R, keep_last=True)
+    returned = {}
+    val, odom = b.run_windows(dev_step_factory(dev_scans, frames, returned), W, K, R, keep_last=True)
     launches = (pkg.kernel_launches() - launches0) // R
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, returned["pose"], odom.stats)
     gpu_poses = odom.poses()
     gpu_frames = list(frames)
     map_voxels, map_points = odom.local_map().size()

@@ -8,8 +8,8 @@ against them, so parity is pinned to reference outputs even where oracle/_ref ca
 Two families:
   fixtures_hash_map_test.npz  the six known-answer inputs of L/src/tests/hash_map_test.hpp (the reference's
                               only tests, SURVEY section 4) with the reference's outputs on them;
-  fixtures_path.npz           seeded synthetic inputs through every function of the hot path
-                              (SURVEY section 8a rows a1-a19) with the reference's outputs;
+  fixtures_path_<i>.npz       seeded synthetic inputs through every function of the hot path
+                              (SURVEY section 8a rows a1-a19) with the reference's outputs, in parts under 1 MB;
   fixtures_frame.npz          seeded PointCloud2 payloads through frame::Lidar::process_frame (SURVEY section 8f N3).
 Regenerate a subset with:  python tests/golden/make_golden.py frame
 """
@@ -166,8 +166,9 @@ def path_fixtures(ref):
     curv[0] = 0.37
     ixyz = (rng.normal(size=(nimu, 3)) * 25).astype(np.float32)
     pil = np.array([0.1, -0.05, 0.2])
-    r = ref.imu_deskew_reference(ixyz, curv, imu, t0, [0.3, -0.2, 9.81], pil, [0.001, 0.002, -0.001])
-    out.update(imu_xyz=ixyz, imu_curv=curv, imu_table=r["table"], imu_rot_end=r["rot_end"], imu_pos_lidar_end=r["pos_lidar_end"], imu_pil=pil,
+    mean_acc, bg = np.array([0.3, -0.2, 9.81]), np.array([0.001, 0.002, -0.001])
+    r = ref.imu_deskew_reference(ixyz, curv, imu, t0, mean_acc, pil, bg)
+    out.update(imu_samples=imu, imu_t0=t0, imu_mean_acc=mean_acc, imu_bg=bg, imu_xyz=ixyz, imu_curv=curv, imu_table=r["table"], imu_rot_end=r["rot_end"], imu_pos_lidar_end=r["pos_lidar_end"], imu_pil=pil,
                imu_deskewed=r["deskewed"], imu_written_back=r["written_back"])
     # KissICP sequence (register_frame x 6, deskew on), scans from the package's own generator
     import __graft_entry__ as g
@@ -230,6 +231,27 @@ def ekf_fixtures():
             "P": np.array([states[i][1] for i in idx])}
 
 
+def save_parts(stem, arrays, max_bytes=900_000):
+    """Write `arrays` (in order) as stem_0.npz, stem_1.npz, ...: a new part starts before max_bytes of array data, so no stored file
+    reaches 1 MB. tests/test_golden.py merges the parts back into one mapping."""
+    for f in os.listdir(HERE):
+        if f.startswith(stem + "_") and f.endswith(".npz"):
+            os.remove(os.path.join(HERE, f))
+    parts, size = [{}], 0
+    for k, v in arrays.items():
+        v = np.asarray(v)
+        if parts[-1] and size + v.nbytes > max_bytes:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += v.nbytes
+    names = [f"{stem}_{i}.npz" for i in range(len(parts))]
+    for name, part in zip(names, parts):
+        np.savez_compressed(os.path.join(HERE, name), **part)
+        assert os.path.getsize(os.path.join(HERE, name)) < 1 << 20, f"{name}: one array of {list(part)} alone reaches 1 MB; sample it"
+    return names
+
+
 if __name__ == "__main__":
     oracle.build_ref()
     ref = oracle.load_ref()
@@ -239,8 +261,7 @@ if __name__ == "__main__":
         np.savez_compressed(os.path.join(HERE, "fixtures_hash_map_test.npz"), **hash_map_test_fixtures(ref))
         made.append("fixtures_hash_map_test.npz")
     if "path" in which:
-        np.savez_compressed(os.path.join(HERE, "fixtures_path.npz"), **path_fixtures(ref))
-        made.append("fixtures_path.npz")
+        made += save_parts("fixtures_path", path_fixtures(ref))
     if "frame" in which:
         np.savez_compressed(os.path.join(HERE, "fixtures_frame.npz"), **frame_fixtures(ref))
         made.append("fixtures_frame.npz")

@@ -65,6 +65,25 @@ def test_forward_pass_matches_the_reference_ekf(pkg, ref, port, rng, case):
     assert np.all(np.abs(wb - r["written_back"]) <= ulp) and (wb != r["written_back"]).mean() < 1e-3
 
 
+def test_forward_pass_matches_golden_table(pkg, port):
+    """The same checks against the reference's outputs recorded by tests/golden/make_golden.py on its IMU window (22 samples at 200 Hz,
+    turning and accelerating platform) with the scan start, mean acceleration and gyro bias stored beside it: no compiled reference needed."""
+    from test_golden import PA
+    t0 = float(PA["imu_t0"])
+    st = make_state(pkg, PA["imu_mean_acc"], PA["imu_pil"], PA["imu_bg"], 0.0, PA["imu_table"][0])
+    curv = PA["imu_curv"]
+    table, rot_end, ple = pkg.imu_forward_pass(st, PA["imu_samples"], t0, float(curv[-1]))
+    assert table.shape == PA["imu_table"].shape
+    np.testing.assert_allclose(table, PA["imu_table"], rtol=0, atol=1e-12)
+    np.testing.assert_allclose(rot_end, PA["imu_rot_end"], rtol=0, atol=1e-12)
+    np.testing.assert_allclose(ple, PA["imu_pos_lidar_end"], rtol=0, atol=1e-12)
+    assert st.last_lidar_end_time == t0 + float(curv[-1]) / 1000.0
+    assert np.array_equal(np.array(st.acc_s_last), table[-1, 1:4]) and np.array_equal(np.array(st.ang_vel_last), table[-1, 4:7])
+    out, wb = port.deskew_imu(PA["imu_xyz"], curv, table, rot_end, ple, PA["imu_pil"])
+    ulp = np.spacing(np.abs(PA["imu_written_back"]).astype(np.float32))
+    assert np.all(np.abs(wb - PA["imu_written_back"]) <= ulp) and (wb != PA["imu_written_back"]).mean() < 1e-3
+
+
 def _random_seeds_n():
     """4 seeds in the suite; LIMU_RANDOM_SEEDS_N="lo-hi" widens the campaign (profiles/r2_random_campaign.json)."""
     import os
