@@ -103,8 +103,10 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
-// The 16 sums one gated correspondence adds to (registration.cpp:46-58,75-76); zeros when gated out.
-__device__ __forceinline__ void contribution(double *c, const V3 &s, const V3 &t, double d2, double th, bool on) {
+// The 16 sums one gated correspondence adds to (registration.cpp:46-58,75-76); zeros when gated out. A gated-out query's
+// coordinates are replaced by zeros too: weight 0 times a NaN or infinite source would be NaN and poison the normal equations.
+__device__ __forceinline__ void contribution(double *c, const V3 &s_in, const V3 &t_in, double d2, double th, bool on) {
+    const V3 s = on ? s_in : V3{0.0, 0.0, 0.0}, t = on ? t_in : V3{0.0, 0.0, 0.0};
     const double rx = s.x - t.x, ry = s.y - t.y, rz = s.z - t.z;       // residual = source - target (:48)
     const double den = th + d2;
     const double w = on ? (th * th) / (den * den) : 0.0;                // :57-58

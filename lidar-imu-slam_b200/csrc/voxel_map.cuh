@@ -57,9 +57,17 @@ __host__ __device__ __forceinline__ int block_stride(int cap) { return (2 + 3 * 
 __host__ __device__ __forceinline__ Slot *slot_at(const MapView &m, unsigned int slot) { return reinterpret_cast<Slot *>(m.blk + (size_t)slot * (size_t)m.stride); }
 __device__ __forceinline__ double *voxel_rows(const MapView &m, unsigned int slot) { return m.blk + (size_t)slot * (size_t)m.stride + 2; }
 
-// utils::get_vox_index, calculation_helpers.cpp:142-147: IEEE double division, truncation toward zero.
-__device__ __forceinline__ int vox_index(double p, double v) { return __double2int_rz(p / v); }
-__device__ __forceinline__ int vox_index(const MapView &m, double p) { return __double2int_rz(m.inv_vox != 0.0 ? p * m.inv_vox : p / m.vox); }
+// utils::get_vox_index, calculation_helpers.cpp:142-147: IEEE double division, truncation toward zero, with the x86-64 semantics of
+// the reference's (int) cast (cvttsd2si): a NaN quotient, or one whose truncation leaves int32, gives INT_MIN. cvt.rzi alone would give 0
+// for NaN (aliasing a real voxel) and saturate beyond int32. INT_MIN lies outside the packed key range, so lookups see "absent" and the
+// entries that make keys report LIMU_ERR_KEY_RANGE without a test of their own.
+constexpr int VOX_INDEX_INVALID = -2147483647 - 1;
+__device__ __forceinline__ int vox_trunc(double q) {
+    // |q| >= 2^31: the saturated -2^31 is INT_MIN already, +2^31 and beyond become INT_MIN; NaN fails the compare
+    return fabs(q) < 2147483648.0 ? __double2int_rz(q) : VOX_INDEX_INVALID;
+}
+__device__ __forceinline__ int vox_index(double p, double v) { return vox_trunc(p / v); }
+__device__ __forceinline__ int vox_index(const MapView &m, double p) { return vox_trunc(m.inv_vox != 0.0 ? p * m.inv_vox : p / m.vox); }
 
 __device__ __forceinline__ bool key_in_range(int x, int y, int z) {
     return (unsigned)(x + KEY_BIAS - 1) < (unsigned)(2 * KEY_BIAS - 1) && (unsigned)(y + KEY_BIAS - 1) < (unsigned)(2 * KEY_BIAS - 1) &&
@@ -633,7 +641,7 @@ __device__ __forceinline__ int voxel_normal(const MapView &m, int slot, int c, d
 __device__ __forceinline__ unsigned int insert_claim_one(const MapView &m, const V3 &p, unsigned int i, unsigned long long birth_base, DevStatus *st, bool *claimed) {
     const int kx = vox_index(m, p.x), ky = vox_index(m, p.y), kz = vox_index(m, p.z);
     unsigned int slot = PEND_NONE;
-    if (!key_in_range(kx, ky, kz) || p.x != p.x || p.y != p.y || p.z != p.z) { st->key_range = 1; return slot; }   // NaN -> INT_MIN in the reference
+    if (!key_in_range(kx, ky, kz)) { st->key_range = 1; return slot; }   // (NaN gives INT_MIN: out of range)
     const unsigned long long key = pack_key(kx, ky, kz);
     unsigned int s = slot_of(key, m.shift);
     for (unsigned int probes = 0; probes <= m.mask; ++probes) {
@@ -694,12 +702,14 @@ __device__ __forceinline__ void insert_place_one(const MapView &m, const V3 &p, 
 // remove_points_from_far (voxel_hash_map.cpp:146-171) as it executes under null locks, for slot s: voxels whose INDEX
 // distance^2 to the origin voxel exceeds max_distance^2 (units as written, :148,:160) drop their points farther than
 // max_distance metres from origin, order preserved (voxel_block.cpp:107-118); empty voxels are erased (tombstoned).
-// the voxel test of :160 on a packed key (origin voxel ovx/ovy/ovz)
+// the voxel test of :160 on a packed key (origin voxel ovx/ovy/ovz). Vector3i::squaredNorm() is int arithmetic: the difference and
+// the sum of squares wrap modulo 2^32, so a voxel ~46 341 or more indices away can pass for a near one and survive. Reproduced on
+// purpose (map contents stay bit-exact with the reference), in unsigned arithmetic so that the wrap is defined behaviour.
 __device__ __forceinline__ bool voxel_is_far(unsigned long long key, int ovx, int ovy, int ovz, double max_sq) {
     int x, y, z;
     unpack_key(key, x, y, z);
-    const long long dx = x - ovx, dy = y - ovy, dz = z - ovz;
-    const long long d2 = dx * dx + dy * dy + dz * dz;
+    const unsigned dx = (unsigned)x - (unsigned)ovx, dy = (unsigned)y - (unsigned)ovy, dz = (unsigned)z - (unsigned)ovz;
+    const int d2 = (int)(dx * dx + dy * dy + dz * dz);
     return (double)d2 > max_sq;
 }
 // returns true when the voxel was erased

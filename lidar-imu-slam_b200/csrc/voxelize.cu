@@ -75,8 +75,8 @@ __device__ __forceinline__ Claim claim_issue(unsigned long long *keys, int shift
     c.valid = false; c.key = KEY_EMPTY; c.cur = KEY_EMPTY; c.s = 0u;
     if (active) {
         const int kx = vox_index(p.x, vs), ky = vox_index(p.y, vs), kz = vox_index(p.z, vs);
-        // NaN: the reference's (int) cast gives INT_MIN on x86-64 (cvttsd2si), far outside the packed range; cvt.rzi gives 0
-        if (!key_in_range(kx, ky, kz) || p.x != p.x || p.y != p.y || p.z != p.z) st->key_range = 1;
+        // NaN: the reference's (int) cast gives INT_MIN on x86-64 (cvttsd2si), and so does vox_index: far outside the packed range
+        if (!key_in_range(kx, ky, kz)) st->key_range = 1;
         else {
             c.valid = true;
             c.key = pack_key(kx, ky, kz);

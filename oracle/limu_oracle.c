@@ -307,8 +307,10 @@ void lo_map_remove_far(lo_map *m, const double *origin) {
     for (long e = 0; e < m->n_entries; ++e) {
         if (m->counts[e] < 0) continue;
         const int *k = m->keys + 3 * e;
-        const int dx = k[0] - ov[0], dy = k[1] - ov[1], dz = k[2] - ov[2];
-        const int d2 = dx * dx + dy * dy + dz * dz; /* Vector3i squaredNorm: int arithmetic */
+        /* Vector3i squaredNorm: int arithmetic, which wraps modulo 2^32 in the reference's build; written unsigned so that the wrap is
+         * defined behaviour here rather than signed overflow */
+        const uint32_t dx = (uint32_t)k[0] - (uint32_t)ov[0], dy = (uint32_t)k[1] - (uint32_t)ov[1], dz = (uint32_t)k[2] - (uint32_t)ov[2];
+        const int d2 = (int)(dx * dx + dy * dy + dz * dz);
         if ((double)d2 > max_dist_sq) {
             double *p = m->pts + 3 * (size_t)e * (size_t)m->cap;
             int w = 0;

@@ -11,6 +11,33 @@ def np_keys(xyz, s):
     return np.trunc(xyz / s).astype(np.int64)
 
 
+def np_vox_index_x86(xyz, s):
+    """get_vox_index as the reference's x86-64 build executes it: (int)(p / v) is cvttsd2si, which gives INT_MIN where the
+    quotient is NaN or its truncation leaves int32."""
+    q = np.asarray(xyz, np.float64) / s
+    ok = (q > -2147483649.0) & (q < 2147483648.0)
+    return np.where(ok, np.trunc(np.where(ok, q, 0.0)), -2147483648.0).astype(np.int32)
+
+
+def np_remove_far(keys, counts, pts, origin, vox, max_distance):
+    """VoxelHashMap::remove_points_from_far (voxel_hash_map.cpp:146-171) on a dump (keys [V,3] int32, counts [V], pts): a voxel whose
+    Vector3i::squaredNorm() distance to the origin's voxel exceeds max_distance^2 drops its points farther than max_distance from
+    origin (order kept) and disappears when none is left. squaredNorm is int arithmetic: the subtraction and the sum of squares wrap
+    modulo 2^32 (a voxel ~46 341 indices away can survive). -> the dump after the eviction."""
+    ov = np_vox_index_x86(np.asarray(origin, np.float64).reshape(1, 3), vox)[0]
+    d = keys.astype(np.uint32) - ov.astype(np.uint32)
+    d2 = (d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1] + d[:, 2] * d[:, 2]).view(np.int32)
+    max_sq = float(max_distance) * float(max_distance)
+    far_voxel = d2.astype(np.float64) > max_sq
+    owner = np.repeat(np.arange(len(keys)), counts)
+    a = pts - np.asarray(origin, np.float64)
+    far_point = ((a[:, 0] * a[:, 0] + a[:, 1] * a[:, 1]) + a[:, 2] * a[:, 2]) > max_sq
+    keep = ~(far_voxel[owner] & far_point)
+    new_counts = np.bincount(owner[keep], minlength=len(keys)).astype(np.int32)
+    alive = new_counts > 0
+    return keys[alive], new_counts[alive], pts[keep]
+
+
 def np_pack(k):
     return ((k[:, 0] + BIAS) << 42) | ((k[:, 1] + BIAS) << 21) | (k[:, 2] + BIAS)
 
