@@ -253,10 +253,7 @@ int limu_odom_register_frame_dev(limu_odom *o, const float *xyzt_dev, int64_t n,
  * (the twist of a scan prepared ahead is taken by the device's log instead of the host's: ~1e-15). */
 int limu_odom_hint_next_dev(limu_odom *o, const float *xyzt_dev_next, int64_t n_next);
 /* Handle options. LIMU_OPT_SPECULATE (default 1; the environment variable LIMU_SPECULATE=0 changes the default): see above.
- * LIMU_OPT_CLUSTER_LOOP (default 0; LIMU_CLUSTER_LOOP=1): with the reference's registration rules the Gauss-Newton loop of a scan runs on
- * ONE 16-CTA thread-block cluster (rows exchanged through distributed shared memory, hardware cluster barrier) instead of ~70 CTAs that
- * meet at a global-memory barrier. Same results; measured SLOWER on B200 (13.5 vs 10.4 us per iteration: the exchange shrinks from 3.5
- * to 1.2 us, but 16 SMs issue the ~2.4 k lookups of an iteration 3.5x slower than 72 SMs do), so it is an opt-in experiment. */
+ * LIMU_OPT_CLUSTER_LOOP: retired, accepted and ignored -- the loop shape it selected gave the same results more slowly (DESIGN.md section 9). */
 enum { LIMU_OPT_SPECULATE = 1, LIMU_OPT_CLUSTER_LOOP = 2 };
 int limu_odom_set_option(limu_odom *o, int32_t option, int64_t value);
 /* Wait for everything the handle has in flight (a map update, kernels launched ahead for a hinted scan) and return the status of a map

@@ -573,7 +573,7 @@ class KissICP:
     """lidar::KissICP (sensors/lidar/icp.hpp:31-68); config = frame::Lidar::ProcessingInfo fields."""
 
     def __init__(self, ctx, voxel_size=1.0, max_range=100.0, cap=10, deskew=False, min_motion_th=0.1, icp_max_iteration=500,
-                 initial_threshold=2.0, estimation_threshold=1e-4, map_capacity_voxels=0, icp_mode=0, speculate=None, cluster_loop=None):
+                 initial_threshold=2.0, estimation_threshold=1e-4, map_capacity_voxels=0, icp_mode=0, speculate=None):
         self.ctx = ctx
         cfg = OdomConfig()
         lib().limu_odom_default_config(C.byref(cfg))
@@ -589,8 +589,6 @@ class KissICP:
         self.stats = FrameStats()
         if speculate is not None:
             self.set_speculate(speculate)
-        if cluster_loop is not None:
-            _chk(lib().limu_odom_set_option(self.h, 2, int(bool(cluster_loop))))   # LIMU_OPT_CLUSTER_LOOP
 
     def set_speculate(self, on: bool):
         """LIMU_OPT_SPECULATE: pipeline consecutive scans when the next one is known (hint_next_dev / prefetch; see limu_cuda.h)."""

@@ -22,7 +22,6 @@ struct FrameFusion {
     DevStatus *status;         // the frame kernel's status word (per odometry handle); nullptr = the context's
     cudaStream_t stream;       // where to launch (nullptr: the context's stream)
     unsigned int *barrier;     // 8 zero-at-rest words private to the caller for the grid barriers (nullptr: the context's; launches on different streams need their own)
-    int allow_cluster;         // LIMU_OPT_CLUSTER_LOOP: the cluster latency shape may be used (registration.cu, k_frame_cluster)
 };
 }  // namespace limu
 struct limu_map;

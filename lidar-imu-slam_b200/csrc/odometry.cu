@@ -87,7 +87,6 @@ struct limu_odom {
     int64_t pf_n[2] = {-1, -1};
     uint64_t pf_seq[2] = {0, 0}, pf_counter = 0;   // order in which the pending uploads were requested
     cudaEvent_t clouds_done = nullptr;
-    bool cluster_loop = false;              // LIMU_OPT_CLUSTER_LOOP: run the Gauss-Newton loop on one 16-CTA cluster (registration.cu, k_frame_cluster); measured slower, opt-in; plain path only
     // ---- pipelined path (LIMU_OPT_SPECULATE, on by default; packed float4 scans) -------------------------------------------------------
     // When the library knows which scan comes next (a device-pointer hint from limu_odom_hint_next_dev, or the scan limu_odom_prefetch is
     // uploading) the work of consecutive scans overlaps on the device and with the host:
@@ -299,7 +298,6 @@ static int odom_register_device(limu_odom *o, const void *raw_dev, int mode, int
     fuse.iqr_in = o->src0[par].as<double>(); fuse.iqr_n = counts + 1; fuse.iqr_d2 = o->d2.as<double>(); fuse.iqr_out = o->src[par].as<double>(); fuse.iqr_count = cnt + 2;
     fuse.upd_down = o->down[par].as<double>(); fuse.upd_n = counts + 0; fuse.upd_world = o->world.as<double>(); fuse.upd_pslot = o->map->pslot.as<unsigned int>();
     fuse.upd_birth_base = o->map->birth_base;
-    fuse.allow_cluster = o->cluster_loop ? 1 : 0;
     fuse.status = res_update_status(cnt, par);
     pose_store(last, fuse.last_pose);
     const int64_t upper_before = o->map->used_upper;
@@ -612,7 +610,6 @@ int limu_odom_create(limu_ctx *c, const limu_odom_config *cfg, limu_odom **out) 
     o->ctx = c;
     o->cfg = *cfg;
     if (const char *e = getenv("LIMU_SPECULATE")) o->speculate = atoi(e) != 0;        // default of LIMU_OPT_SPECULATE (on)
-    if (const char *e = getenv("LIMU_CLUSTER_LOOP")) o->cluster_loop = atoi(e) != 0;   // default of LIMU_OPT_CLUSTER_LOOP (off)
     int64_t capv = cfg->map_capacity_voxels;
     if (capv <= 0) {   // a sensor sees a shell, not a ball: ~ (2 r / v)^2 * 8 voxels is generous for one neighbourhood
         const double side = 2.0 * cfg->max_range / cfg->voxel_size;
@@ -835,7 +832,7 @@ int limu_odom_set_option(limu_odom *o, int32_t option, int64_t value) {
         if (!o->speculate) { o->hint_ptr = nullptr; o->hint_n = 0; }
         return st;
     }
-    if (option == LIMU_OPT_CLUSTER_LOOP) { o->cluster_loop = value != 0; return LIMU_OK; }
+    if (option == LIMU_OPT_CLUSTER_LOOP) return LIMU_OK;   // retired: accepted and ignored (limu_cuda.h)
     set_error("limu_odom_set_option: unknown option %d", (int)option);
     return LIMU_ERR_INVALID;
 }

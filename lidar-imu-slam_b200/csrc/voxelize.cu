@@ -14,8 +14,6 @@
 // this launch is un-claimed by the NEXT launch, which works on the other of two stage-2 tables.
 // "First point per voxel wins, output in first-occurrence order" (icp.cpp:13-27 + the oracle's ordered map) becomes:
 // atomicMin of the input index per voxel, then a stable compaction over VX_BLOCK-point tiles.
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "compact.cuh"
@@ -27,15 +25,9 @@ LIMU_TRACE_RING(limu_debug_trace_vox)
 
 namespace limu {
 
-#ifndef LIMU_VX_BLOCK
-#define LIMU_VX_BLOCK 1024   // one fat CTA per SM: a grid barrier is paid per ARRIVING CTA (atomics on one word serialise at ~4 ns each: 592 CTAs of 256 -> 148 of 1024)
-#endif
-constexpr int VX_BLOCK = LIMU_VX_BLOCK;
-// The pipelined odometry path (odometry.cu) runs the NEXT scan's launch beside the current scan's map update: 1024 threads x 64 registers
-// are a whole register file, so that launch uses half-size CTAs (one per SM) and leaves room for the update kernel's CTA.
-constexpr int VX_BLOCK_BESIDE = 512;
-constexpr int VX_TILE = 1024;            // points per tile in both shapes (1024 x 1 and 512 x 2)
-static_assert(VX_BLOCK == VX_TILE, "the full-size launch handles one point per thread");
+// Threads per CTA and points per tile (one point per thread). One fat CTA per SM: a grid barrier is paid per ARRIVING CTA (atomics on one
+// word serialise at ~4 ns each: 592 CTAs of 256 -> 148 of 1024).
+constexpr int VX_BLOCK = 1024;
 
 struct VoxelizeArgs {
     const void *raw;            // mode 0: float4 {x,y,z,t}; mode 1: records `stride` bytes apart + ts; mode 2: double xyz (already a frame)
@@ -61,39 +53,20 @@ struct VoxelizeArgs {
     DevStatus *st_next;         // non-null: the status word of the NEXT launch of this pipeline (two words alternate); zeroed late in this launch
 };
 
-// Claim the voxel of p in a scan-local table and note `index` as a candidate for its first point (atomicMin). Split in two so that a thread
-// with several points has all their first probes in flight together: claim_issue sends ONE compare-and-swap per point (it both finds and
-// claims: the slot is the voxel's if it was empty or already held the key), claim_finish looks at the answer and walks on in the rare case
-// of a collision.
-struct Claim {
-    unsigned long long key, cur;
-    unsigned int s;
-    bool valid;
-};
-__device__ __forceinline__ Claim claim_issue(unsigned long long *keys, int shift, const V3 &p, double vs, bool active, DevStatus *st) {
-    Claim c;
-    c.valid = false; c.key = KEY_EMPTY; c.cur = KEY_EMPTY; c.s = 0u;
-    if (active) {
-        const int kx = vox_index(p.x, vs), ky = vox_index(p.y, vs), kz = vox_index(p.z, vs);
-        // NaN: the reference's (int) cast gives INT_MIN on x86-64 (cvttsd2si), and so does vox_index: far outside the packed range
-        if (!key_in_range(kx, ky, kz)) st->key_range = 1;
-        else {
-            c.valid = true;
-            c.key = pack_key(kx, ky, kz);
-            c.s = slot_of(c.key, shift);
-            c.cur = atomicCAS(&keys[c.s], KEY_EMPTY, c.key);
-        }
-    }
-    return c;
-}
-__device__ __forceinline__ unsigned int claim_finish(const Claim &c, unsigned long long *keys, unsigned int *minidx, unsigned int mask, unsigned int index, DevStatus *st) {
-    if (!c.valid) return PEND_NONE;
-    unsigned int s = c.s;
-    unsigned long long cur = c.cur;
+// Claim the voxel of p in a scan-local table and note `index` as a candidate for its first point (atomicMin). Each probe is ONE
+// compare-and-swap that both finds and claims: the slot is the voxel's if it was empty or already held the key. Returns the slot, or
+// PEND_NONE for a key out of range or a full table (both reported in *st).
+__device__ __forceinline__ unsigned int claim(unsigned long long *keys, unsigned int *minidx, int shift, unsigned int mask, const V3 &p, double vs,
+                                              unsigned int index, DevStatus *st) {
+    const int kx = vox_index(p.x, vs), ky = vox_index(p.y, vs), kz = vox_index(p.z, vs);
+    // NaN: the reference's (int) cast gives INT_MIN on x86-64 (cvttsd2si), and so does vox_index: far outside the packed range
+    if (!key_in_range(kx, ky, kz)) { st->key_range = 1; return PEND_NONE; }
+    const unsigned long long key = pack_key(kx, ky, kz);
+    unsigned int s = slot_of(key, shift);
     for (unsigned int probes = 0; probes <= mask; ++probes) {
-        if (cur == KEY_EMPTY || cur == c.key) { atomicMin(&minidx[s], index); return s; }
+        const unsigned long long cur = atomicCAS(&keys[s], KEY_EMPTY, key);
+        if (cur == KEY_EMPTY || cur == key) { atomicMin(&minidx[s], index); return s; }
         s = (s + 1) & mask;
-        cur = atomicCAS(&keys[s], KEY_EMPTY, c.key);
     }
     st->table_full = 1;
     return PEND_NONE;
@@ -153,17 +126,14 @@ __device__ unsigned long long g_vox_marks[8];   // globaltimer of thread 0 of CT
 #define VX_MARK(k) do {} while (0)
 #endif
 
-// BLOCK threads handle tiles of VX_TILE = BLOCK * ITEMS consecutive points, ITEMS per thread: the full-size launch is 1024 x 1, the launch
-// that runs beside the map update 512 x 2 -- half the registers per SM, the same tiles, and a thread's two claims in flight together.
-template <int BLOCK, int ITEMS>
+// VX_BLOCK threads handle tiles of VX_BLOCK consecutive points, one point per thread.
 __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
-    constexpr int TILE = BLOCK * ITEMS;
     __shared__ int ws[32];
     __shared__ int total;
     GridSync gs{A.barrier, 0u, gridDim.x};
     const int64_t n = A.n;
-    const int64_t gtid = (int64_t)blockIdx.x * BLOCK + threadIdx.x, gthreads = (int64_t)gridDim.x * BLOCK;
-    const int ntiles = (int)((n + TILE - 1) / TILE);
+    const int64_t gtid = (int64_t)blockIdx.x * VX_BLOCK + threadIdx.x, gthreads = (int64_t)gridDim.x * VX_BLOCK;
+    const int ntiles = (int)((n + VX_BLOCK - 1) / VX_BLOCK);
     VX_MARK(0);
     LIMU_TRACE(10);
     // un-claim what the previous launch left in ITS stage-2 table (this launch uses the other one): no barrier needed
@@ -185,80 +155,50 @@ __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
                 for (int k = 0; k < 6; ++k) tw[k] = __ldcg(A.twist_dev + k);
             }
         }
-        for (int64_t i0 = gtid; i0 < n; i0 += (int64_t)ITEMS * gthreads) {
-            V3 p[ITEMS];
-            Claim c[ITEMS];
-#pragma unroll
-            for (int u = 0; u < ITEMS; ++u) {
-                const int64_t i = i0 + (int64_t)u * gthreads;
-                const bool on = i < n;
-                double t = 0.0;
-                p[u] = V3{0.0, 0.0, 0.0};
-                if (on) {
-                    if (A.mode == 0) {
-                        const float4 q = __ldg(reinterpret_cast<const float4 *>(A.raw) + i);
-                        p[u] = V3{(double)q.x, (double)q.y, (double)q.z};
-                        t = (double)q.w;
-                    } else if (A.mode == 1) {
-                        const float *q = reinterpret_cast<const float *>(static_cast<const unsigned char *>(A.raw) + (size_t)i * A.stride);
-                        p[u] = V3{(double)q[0], (double)q[1], (double)q[2]};
-                        if (A.deskew) t = A.ts[i];
-                    } else {
-                        const double *q = static_cast<const double *>(A.raw) + 3 * i;
-                        p[u] = V3{q[0], q[1], q[2]};
-                    }
-                    if (A.deskew) {
-                        const double s = t - 0.5;   // mid_pose_timestamp, deskew.hpp:12
-                        double st[6];
-#pragma unroll
-                        for (int k = 0; k < 6; ++k) st[k] = s * tw[k];
-                        p[u] = apply(se3_exp(st), p[u]);
-                    }
-                    A.frame[3 * i] = p[u].x; A.frame[3 * i + 1] = p[u].y; A.frame[3 * i + 2] = p[u].z;
-                }
-                c[u] = claim_issue(A.keys1, A.shift1, p[u], A.vs1, on, A.st);
+        for (int64_t i = gtid; i < n; i += gthreads) {
+            double t = 0.0;
+            V3 p;
+            if (A.mode == 0) {
+                const float4 q = __ldg(reinterpret_cast<const float4 *>(A.raw) + i);
+                p = V3{(double)q.x, (double)q.y, (double)q.z};
+                t = (double)q.w;
+            } else if (A.mode == 1) {
+                const float *q = reinterpret_cast<const float *>(static_cast<const unsigned char *>(A.raw) + (size_t)i * A.stride);
+                p = V3{(double)q[0], (double)q[1], (double)q[2]};
+                if (A.deskew) t = A.ts[i];
+            } else {
+                const double *q = static_cast<const double *>(A.raw) + 3 * i;
+                p = V3{q[0], q[1], q[2]};
             }
+            if (A.deskew) {
+                const double s = t - 0.5;   // mid_pose_timestamp, deskew.hpp:12
+                double st[6];
 #pragma unroll
-            for (int u = 0; u < ITEMS; ++u) {
-                const int64_t i = i0 + (int64_t)u * gthreads;
-                if (i < n) A.pslot1[i] = claim_finish(c[u], A.keys1, A.min1, A.mask1, (unsigned int)i, A.st);
+                for (int k = 0; k < 6; ++k) st[k] = s * tw[k];
+                p = apply(se3_exp(st), p);
             }
+            A.frame[3 * i] = p.x; A.frame[3 * i + 1] = p.y; A.frame[3 * i + 2] = p.z;
+            A.pslot1[i] = claim(A.keys1, A.min1, A.shift1, A.mask1, p, A.vs1, (unsigned int)i, A.st);
         }
     }
     gs.sync();
     VX_MARK(1);
     LIMU_TRACE(11);
     // P2: a point survives stage 1 iff it holds its voxel's smallest input index. Per tile: flags, count (published), ordered scatter
-    // -> down[]; each winner immediately claims its 1.5 v voxel with its OUTPUT index. A thread owns ITEMS consecutive points of the tile.
+    // -> down[]; each winner immediately claims its 1.5 v voxel with its OUTPUT index.
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int64_t e0 = (int64_t)tile * TILE + (int64_t)threadIdx.x * ITEMS;
-        int f[ITEMS], cnt = 0;
-#pragma unroll
-        for (int u = 0; u < ITEMS; ++u) {
-            const int64_t i = e0 + u;
-            f[u] = 0;
-            if (i < n) { const unsigned int s = A.pslot1[i]; f[u] = s != PEND_NONE && __ldcg(A.min1 + s) == (unsigned int)i; }
-            cnt += f[u];
-        }
-        const int r = block_exclusive_scan_count(cnt, &total, ws);
+        const int64_t i = (int64_t)tile * VX_BLOCK + threadIdx.x;
+        int f = 0;
+        if (i < n) { const unsigned int s = A.pslot1[i]; f = s != PEND_NONE && __ldcg(A.min1 + s) == (unsigned int)i; }
+        const int r = block_exclusive_scan_count(f, &total, ws);
         if (threadIdx.x == 0) tile_publish(A.tile1 + tile, A.epoch, total);
-        const int base = tile_base<BLOCK>(A.tile1, tile, A.epoch, ws);
-        V3 p[ITEMS];
-        Claim c[ITEMS];
-        int j = base + r;
-#pragma unroll
-        for (int u = 0; u < ITEMS; ++u) {
-            const int64_t i = e0 + u;
-            p[u] = V3{0.0, 0.0, 0.0};
-            if (f[u]) {
-                p[u] = V3{A.frame[3 * i], A.frame[3 * i + 1], A.frame[3 * i + 2]};
-                A.down[3 * (size_t)(j + (u ? f[0] : 0))] = p[u].x; A.down[3 * (size_t)(j + (u ? f[0] : 0)) + 1] = p[u].y; A.down[3 * (size_t)(j + (u ? f[0] : 0)) + 2] = p[u].z;
-            }
-            c[u] = claim_issue(A.keys2, A.shift2, p[u], A.vs2, f[u] != 0, A.st);
+        const int base = tile_base<VX_BLOCK>(A.tile1, tile, A.epoch, ws);
+        if (f) {
+            const int j = base + r;
+            const V3 p{A.frame[3 * i], A.frame[3 * i + 1], A.frame[3 * i + 2]};
+            A.down[3 * (size_t)j] = p.x; A.down[3 * (size_t)j + 1] = p.y; A.down[3 * (size_t)j + 2] = p.z;
+            A.pslot2[j] = claim(A.keys2, A.min2, A.shift2, A.mask2, p, A.vs2, (unsigned int)j, A.st);
         }
-#pragma unroll
-        for (int u = 0; u < ITEMS; ++u)
-            if (f[u]) { const int jj = j + (u ? f[0] : 0); A.pslot2[jj] = claim_finish(c[u], A.keys2, A.min2, A.mask2, (unsigned int)jj, A.st); }
         if (tile == ntiles - 1 && threadIdx.x == 0) { A.counts[0] = base + total; *A.nd_this = base + total; }
         __syncthreads();
     }
@@ -274,26 +214,18 @@ __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
     }
     // P3: the same flag -> count -> scatter over down[] for stage 2
     const int nd = __ldcg(A.counts);
-    const int ntiles2 = (nd + TILE - 1) / TILE;
+    const int ntiles2 = (nd + VX_BLOCK - 1) / VX_BLOCK;
     for (int tile = blockIdx.x; tile < ntiles2; tile += gridDim.x) {
-        const int e0 = tile * TILE + (int)threadIdx.x * ITEMS;
-        int f[ITEMS], cnt = 0;
-#pragma unroll
-        for (int u = 0; u < ITEMS; ++u) {
-            const int j = e0 + u;
-            f[u] = 0;
-            if (j < nd) { const unsigned int s = __ldcg(A.pslot2 + j); f[u] = s != PEND_NONE && __ldcg(A.min2 + s) == (unsigned int)j; }
-            cnt += f[u];
-        }
-        const int r = block_exclusive_scan_count(cnt, &total, ws);
+        const int j = tile * VX_BLOCK + (int)threadIdx.x;
+        int f = 0;
+        if (j < nd) { const unsigned int s = __ldcg(A.pslot2 + j); f = s != PEND_NONE && __ldcg(A.min2 + s) == (unsigned int)j; }
+        const int r = block_exclusive_scan_count(f, &total, ws);
         if (threadIdx.x == 0) tile_publish(A.tile2 + tile, A.epoch, total);
-        const int base = tile_base<BLOCK>(A.tile2, tile, A.epoch, ws);
-#pragma unroll
-        for (int u = 0; u < ITEMS; ++u)
-            if (f[u]) {
-                const size_t k = (size_t)(base + r + (u ? f[0] : 0)), j = (size_t)(e0 + u);
-                A.src0[3 * k] = __ldcg(A.down + 3 * j); A.src0[3 * k + 1] = __ldcg(A.down + 3 * j + 1); A.src0[3 * k + 2] = __ldcg(A.down + 3 * j + 2);
-            }
+        const int base = tile_base<VX_BLOCK>(A.tile2, tile, A.epoch, ws);
+        if (f) {
+            const size_t k = (size_t)(base + r);
+            A.src0[3 * k] = __ldcg(A.down + 3 * (size_t)j); A.src0[3 * k + 1] = __ldcg(A.down + 3 * (size_t)j + 1); A.src0[3 * k + 2] = __ldcg(A.down + 3 * (size_t)j + 2);
+        }
         if (tile == ntiles2 - 1 && threadIdx.x == 0) A.counts[1] = base + total;
         __syncthreads();
     }
@@ -307,11 +239,10 @@ __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
         if (atomicAdd(A.barrier + 1, 1u) == gridDim.x - 1) { A.barrier[0] = 0u; A.barrier[1] = 0u; __threadfence(); }
     }
 }
-// The three launch shapes: full (alone on the GPU: 1024 threads x 64 registers = a whole register file), half (512 x 2 points) and lean
-// (1024 x 1 at 48 registers, a few spills) -- the latter two leave 16 K registers per SM to the map update's CTA that runs beside them.
-static __global__ void __launch_bounds__(VX_BLOCK, 1) k_voxelize_full(const VoxelizeArgs A) { voxelize_body<VX_BLOCK, 1>(A); }
-static __global__ void __launch_bounds__(VX_BLOCK_BESIDE, 2) k_voxelize_half(const VoxelizeArgs A) { voxelize_body<VX_BLOCK_BESIDE, VX_TILE / VX_BLOCK_BESIDE>(A); }
-static __global__ void __maxnreg__(48) k_voxelize_lean(const VoxelizeArgs A) { voxelize_body<VX_BLOCK, 1>(A); }
+// The two launch shapes: full (alone on the GPU: 1024 threads x 64 registers = a whole register file) and lean (48 registers, a few
+// spills), which leaves 16 K registers per SM to the map update's CTA that runs beside it in the pipelined odometry path (odometry.cu).
+static __global__ void __launch_bounds__(VX_BLOCK, 1) k_voxelize_full(const VoxelizeArgs A) { voxelize_body(A); }
+static __global__ void __maxnreg__(48) k_voxelize_lean(const VoxelizeArgs A) { voxelize_body(A); }
 
 // One thread that waits until a frame kernel launched EARLIER on another stream has published the pose of its scan (the flag carries that
 // launch's sequence number): the stream it sits in -- the next scan's k_voxelize behind it -- is released the moment the Gauss-Newton loop is
@@ -379,7 +310,7 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     const int64_t C1 = pow2_slots(n), C2 = pow2_slots(n);
     int lg = 0;
     while ((int64_t(1) << lg) < C1) ++lg;
-    const int ntiles = div_up(n, VX_TILE);
+    const int ntiles = div_up(n, VX_BLOCK);
     {   // three tables [u64 key x cap | u32 min-index x cap] at offsets fixed by the ALLOCATED capacity (claimed slots are remembered as indices), all-ones
         // = clean at rest. Whenever one of the buffers is re-allocated the memory of what the previous launch claimed is gone: start over clean.
         bool reset = false;
@@ -443,10 +374,7 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     // CTA of this cooperative launch has been placed, and this launch sits in front of the loop that gate waits for (see icp_device)
     const int grid = (int)std::min<int64_t>(ntiles, beside ? (int64_t)std::max(1, c->sm_count - GATE_SLACK_SMS) : (int64_t)c->sm_count * g_vx_blocks_per_sm);
     void *args[] = {&A};
-    static const int beside_shape = getenv("LIMU_VX_BESIDE") ? atoi(getenv("LIMU_VX_BESIDE")) : 1;   // 1: lean (measured 2.6 % more scans/s than half, profiles/r2_voxelize_beside_ab.json), 0: half
-    if (beside && beside_shape == 1) LIMU_CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_voxelize_lean, dim3(grid), dim3(VX_BLOCK), args, 0, stream));
-    else if (beside) LIMU_CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_voxelize_half, dim3(grid), dim3(VX_BLOCK_BESIDE), args, 0, stream));
-    else LIMU_CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_voxelize_full, dim3(grid), dim3(VX_BLOCK), args, 0, stream));
+    LIMU_CUDA_TRY(cudaLaunchCooperativeKernel(beside ? (const void *)k_voxelize_lean : (const void *)k_voxelize_full, dim3(grid), dim3(VX_BLOCK), args, 0, stream));
     LIMU_LAUNCHED();
     return LIMU_OK;
 }

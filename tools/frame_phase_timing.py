@@ -68,13 +68,9 @@ names = ["iqr", "icp_loop", "insert_claim", "insert_place", "evict_sweep"]
 print({n: round(float(v), 2) for n, v in zip(names, r.mean(axis=0))}, "total_us", round(float(r.sum(axis=1).mean()), 2), "iters/scan", np.mean(iters),
       "icp_us_per_iter", round(float(r[:, 1].mean() / np.mean(iters)), 2))
 cyc = lambda a, b: int(marks[b] - marks[a])
-if os.environ.get("LIMU_CLUSTER_LOOP", "0") not in ("", "0"):
-    print("cluster shape, iteration 2 of the last scan (SM cycles of CTA 0): row reduce + DSMEM push + cluster barrier", cyc(6, 7), "fold", cyc(7, 8), "ldlt", cyc(8, 9), "exp", cyc(9, 10),
-          "| pass of warp 1", cyc(11, 12), "tail of the solver warp", cyc(13, 14))
-else:
-    print("classic shape, iteration 2 of the last scan (SM cycles of CTA 0, 1965 MHz): pass of warp 0", cyc(6, 7), "| pass end -> S1", cyc(7, 11), "| CTA row + grid barrier", cyc(11, 12),
-          "| fold", cyc(12, 8), "| ldlt", cyc(8, 9), "| exp", cyc(9, 10), "| -> S2", cyc(10, 15), "| whole round (pass start -> S2)", cyc(6, 15),
-          "| tail of the solver warp (its own clock)", cyc(13, 14))
+print("iteration 2 of the last scan (SM cycles of CTA 0, 1965 MHz): pass of warp 0", cyc(6, 7), "| pass end -> S1", cyc(7, 11), "| CTA row + grid barrier", cyc(11, 12),
+      "| fold", cyc(12, 8), "| ldlt", cyc(8, 9), "| exp", cyc(9, 10), "| -> S2", cyc(10, 15), "| whole round (pass start -> S2)", cyc(6, 15),
+      "| tail of the solver warp (its own clock)", cyc(13, 14))
 print("rounds of the Gauss-Newton loop (us, CTA 0, mean over scans; nan = fewer rounds):", [round(float(x), 2) for x in np.nanmean(np.array(rounds), axis=0)])
 if vrows:
     print("k_voxelize phases (us; plain launch, 1024-thread CTAs): P1 deskew + claim | P2 flags, counts, scatter, claim 2 | P3 un-claim, flags, counts, scatter:", [round(float(x), 2) for x in np.mean(np.array(vrows), axis=0)], "total", round(float(np.sum(np.mean(np.array(vrows), axis=0))), 2))
