@@ -183,6 +183,8 @@ def lib():
             "limu_odom_register_frame_dev": [_vp, _vp, C.c_int64, _dp, C.POINTER(FrameStats)],
             "limu_odom_prefetch": [_vp, _fp, C.c_int64],
             "limu_odom_prefetch_cloud": [_vp, _vp, C.c_int32, _dp, C.c_int64],
+            "limu_odom_register_cloud_imu": [_vp, _vp, C.c_int32, C.c_int32, C.c_int64, _dp, C.c_int32, _dp, _dp, _dp, _dp, _dp, _lp, _dp, _lp, C.POINTER(FrameStats)],
+            "limu_odom_prefetch_cloud_imu": [_vp, _vp, C.c_int32, C.c_int32, C.c_int64, _dp, C.c_int32, _dp, _dp, _dp],
             "limu_odom_hint_next_dev": [_vp, _vp, C.c_int64],
             "limu_odom_set_option": [_vp, C.c_int32, C.c_int64],
             "limu_odom_flush": [_vp],
@@ -662,6 +664,35 @@ class KissICP:
         if copy:
             return down[: nd.value].copy(), src[: ns.value].copy(), pose
         return down[: nd.value], src[: ns.value], pose
+
+    @staticmethod
+    def _imu_args(table, rot_end, pos_lidar_end, p_imu_lidar):
+        t = np.ascontiguousarray(table, np.float64).reshape(-1, 22)
+        return (t,) + tuple(np.ascontiguousarray(v, np.float64).reshape(n) for v, n in ((rot_end, 9), (pos_lidar_end, 3), (p_imu_lidar, 3)))
+
+    def register_cloud_imu(self, records, stride_bytes, curvature_offset, table, rot_end, pos_lidar_end, p_imu_lidar, copy=True):
+        """EKF::motion_compensation_with_imu + register_frame(Vec3dVector) in one call (limu_odom_register_cloud_imu): records = contiguous point
+        records (float x,y,z first, float curvature in ms at curvature_offset), table = [M,22] pose rows of imu_forward_pass. -> (down, keypoints,
+        pose) in the scan-end lidar frame. With copy=False the clouds are views into pinned buffers that the next call overwrites."""
+        rec = records if isinstance(records, np.ndarray) and records.flags.c_contiguous else np.ascontiguousarray(records)
+        n = rec.nbytes // int(stride_bytes)
+        t, re, pe, pil = self._imu_args(table, rot_end, pos_lidar_end, p_imu_lidar)
+        pose = np.empty(7)
+        down, src = self._out_buffers(n)
+        nd, ns = C.c_int64(0), C.c_int64(0)
+        _chk(lib().limu_odom_register_cloud_imu(self.h, rec.ctypes.data_as(_vp), int(stride_bytes), int(curvature_offset), n, _d(t), len(t), _d(re), _d(pe), _d(pil),
+                                                _d(pose), _d(down), C.byref(nd), _d(src), C.byref(ns), C.byref(self.stats)))
+        if copy:
+            return down[: nd.value].copy(), src[: ns.value].copy(), pose
+        return down[: nd.value], src[: ns.value], pose
+
+    def prefetch_cloud_imu(self, records, stride_bytes, curvature_offset, table, rot_end, pos_lidar_end, p_imu_lidar):
+        """Start the H2D copy of the NEXT cloud (contiguous records, ideally pinned) and its pose table; pass the same records and IMU arguments to
+        the next register_cloud_imu."""
+        assert isinstance(records, np.ndarray) and records.flags.c_contiguous
+        t, re, pe, pil = self._imu_args(table, rot_end, pos_lidar_end, p_imu_lidar)
+        _chk(lib().limu_odom_prefetch_cloud_imu(self.h, records.ctypes.data_as(_vp), int(stride_bytes), int(curvature_offset), records.nbytes // int(stride_bytes),
+                                                _d(t), len(t), _d(re), _d(pe), _d(pil)))
 
     def register_msg(self, data, fields, cfg, message_time, scan_count, max_segments=16):
         """lidar_callback -> estimate_lidar_odometry for one PointCloud2 payload: preprocess + register every segment on the

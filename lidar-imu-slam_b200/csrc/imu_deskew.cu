@@ -1,20 +1,13 @@
 // imu_deskew.cu -- IMU-propagated backward deskew: the per-point loop of kalman::EKF::motion_compensation_with_imu
 // (L/src/kalman/ekf.cpp:420-468; SURVEY section 8f N1). The host IMU forward pass (:315-410) stays where it is (it walks
 // ~20 IMU samples through the EKF state) and hands over its pose table (kalman::Pose6D rows, ekf.hpp:88-105), the
-// scan-end rotation / lidar position (:393-418) and the IMU->lidar lever arm; every point is then independent:
-//   head   = the latest table row (excluding the last) whose offset_time is below the point's time (:422-433)
-//   R_i    = R_head * AngleAxis(dt |w|, w/|w|)                                   (:444, helper.hpp:35-40)
-//   T_ei   = p + v dt + 0.5 a dt^2 + R_i p_IL - p_lidar_end                      (:445)
-//   P_comp = R_end^T (R_i P_i + T_ei), stored back as FLOAT and widened          (:448-468)
-// The reference's serial loop never consumes the first point of the scan (:455-456), so that point is compensated again
-// by every older head below its time; the kernel reproduces that on thread 0.
+// scan-end rotation / lidar position (:393-418) and the IMU->lidar lever arm; every point is then independent. The math
+// (head rule, compensation, the first point's re-visits) is in imu_compensate.cuh, shared with the fused voxelize kernel.
 #include <algorithm>
 
-#include "common.cuh"
+#include "imu_compensate.cuh"
 
 namespace limu {
-
-constexpr int IMU_MAX_ROWS = 96;
 
 struct ImuDeskewArgs {
     unsigned char *rec;      // point records, `stride` bytes apart: float x,y,z at offset 0, float curvature (ms) at `toff`
@@ -26,41 +19,6 @@ struct ImuDeskewArgs {
     double *out;             // n x 3 (optional)
 };
 
-// Eigen::AngleAxisd(dt*|w|, w.normalized()).toRotationMatrix() (Eigen/src/Geometry/AngleAxis.h)
-__device__ __forceinline__ void ang_vel_to_rmat(const double *w, double dt, double *R) {
-    const double z = sqnorm3(w[0], w[1], w[2]);
-    const double nrm = sqrt(z);
-    double ax = w[0], ay = w[1], az = w[2];
-    if (z > 0.0) { ax = w[0] / nrm; ay = w[1] / nrm; az = w[2] / nrm; }
-    const double angle = dt * nrm;
-    const double s = sin(angle), c = cos(angle);
-    const double sx = s * ax, sy = s * ay, sz = s * az;
-    const double cx = (1.0 - c) * ax, cy = (1.0 - c) * ay, cz = (1.0 - c) * az;
-    double tmp;
-    tmp = cx * ay; R[1] = tmp - sz; R[3] = tmp + sz;
-    tmp = cx * az; R[2] = tmp + sy; R[6] = tmp - sy;
-    tmp = cy * az; R[5] = tmp - sx; R[7] = tmp + sx;
-    R[0] = cx * ax + c; R[4] = cy * ay + c; R[8] = cz * az + c;
-}
-
-__device__ __forceinline__ void compensate(const ImuDeskewArgs &A, const double *T /* table row in shared memory */, double t, float *xyz) {
-    const double dt = t - T[0];
-    double Rw[9], Ri[9], t1[3], t2[3];
-    ang_vel_to_rmat(T + 4, dt, Rw);
-    mat3mul(T + 13, Rw, Ri);
-    mat3vec(Ri, A.p_il, t1);
-    const double P[3] = {(double)xyz[0], (double)xyz[1], (double)xyz[2]};
-    mat3vec(Ri, P, t2);
-    double v[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        const double Tei = (((T[10 + a] + T[7 + a] * dt) + (0.5 * T[1 + a]) * (dt * dt)) + t1[a]) - A.pos_lidar_end[a];
-        v[a] = t2[a] + Tei;
-    }
-#pragma unroll
-    for (int a = 0; a < 3; ++a) xyz[a] = (float)((A.rot_end[a] * v[0] + A.rot_end[3 + a] * v[1]) + A.rot_end[6 + a] * v[2]);
-}
-
 static __global__ void __launch_bounds__(256) k_deskew_imu(const ImuDeskewArgs A) {
     __shared__ double tab[IMU_MAX_ROWS * 22];
     for (int k = threadIdx.x; k < A.M * 22; k += blockDim.x) tab[k] = A.table[k];
@@ -69,15 +27,8 @@ static __global__ void __launch_bounds__(256) k_deskew_imu(const ImuDeskewArgs A
     if (i >= A.n) return;
     float *q = reinterpret_cast<float *>(A.rec + (size_t)i * A.stride);
     float xyz[3] = {q[0], q[1], q[2]};
-    const double t = (double)*reinterpret_cast<const float *>(A.rec + (size_t)i * A.stride + A.toff) / 1000.0;   // curvature / double(1000)
-    int h = A.M - 2;
-    while (h >= 0 && !(t > tab[22 * h])) --h;
-    if (h >= 0) {
-        compensate(A, tab + 22 * h, t, xyz);
-        if (i == 0)   // the serial loop re-visits the first point under every older head (:455-456)
-            for (int g = h - 1; g >= 0; --g) if (t > tab[22 * g]) compensate(A, tab + 22 * g, t, xyz);
-        q[0] = xyz[0]; q[1] = xyz[1]; q[2] = xyz[2];
-    }
+    const double t = imu_point_time(A.rec + (size_t)i * A.stride, A.toff);
+    if (imu_deskew_point(tab, A.M, i, t, A.rot_end, A.pos_lidar_end, A.p_il, xyz)) { q[0] = xyz[0]; q[1] = xyz[1]; q[2] = xyz[2]; }
     if (A.out) { A.out[3 * i] = (double)xyz[0]; A.out[3 * i + 1] = (double)xyz[1]; A.out[3 * i + 2] = (double)xyz[2]; }
 }
 

@@ -26,8 +26,16 @@ struct VoxelizeScratch {
     unsigned int epoch = 0;               // launch counter: validates the per-tile count words
     void release() { table.release(); pslot.release(); tiles.release(); cap_slots = pslot_n = 0; parity = 0; st_word = 0; }
 };
+// The IMU deskew of a cloud of point records (limu_deskew_imu's arguments): `table` = M pose rows of 22 doubles in DEVICE memory, the float
+// curvature (ms) of each record at byte offset toff, the scan-end rotation (row-major) and lidar position, the IMU->lidar lever arm.
+struct ImuDeskew {
+    const double *table;
+    int M, toff;
+    double rot_end[9], pos_lidar_end[3], p_il[3];
+};
 // KissICP::deskew_scan + the two voxel_downsample stages of KissICP::voxelize in one cooperative launch.
-// mode 0: raw = float4 {x,y,z,t}; 1: records `stride` bytes apart + FP64 ts; 2: double xyz (register_frame(Vec3dVector)).
+// mode 0: raw = float4 {x,y,z,t}; 1: records `stride` bytes apart + FP64 ts; 2: double xyz (register_frame(Vec3dVector));
+// 3: records `stride` bytes apart, IMU-deskewed as limu_deskew_imu does (`imu`; deskew / twist are not read).
 // twist_dev (speculative launches, odometry.cu): read the deskew twist from device memory instead of twist_host.
 // own_status: THREE status words private to the pipeline that owns `sc` (zero at first use): consecutive launches rotate through them and each
 // launch zeroes the next one late, so a word is clean when its launch starts without a memset per scan; *status_used = which word this launch
@@ -35,7 +43,8 @@ struct VoxelizeScratch {
 // stream: where to enqueue (nullptr = the context's); beside: half-size CTAs, one per SM, so that the launch fits next to another kernel's CTA.
 int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int mode, int stride, const double *ts_dev, int deskew, const double *twist_host,
                     int64_t n, double v, double *frame_dev, double *down_dev, double *src0_dev, int *counts_dev, const double *twist_dev = nullptr,
-                    DevStatus *own_status = nullptr, int *status_used = nullptr, cudaStream_t stream = nullptr, bool beside = false);
+                    DevStatus *own_status = nullptr, int *status_used = nullptr, cudaStream_t stream = nullptr, bool beside = false,
+                    const ImuDeskew *imu = nullptr);
 // One-thread kernel on stream s that returns once *flag has reached seq (voxelize.cu).
 int gate_device(cudaStream_t s, const unsigned int *flag, unsigned int seq);
 

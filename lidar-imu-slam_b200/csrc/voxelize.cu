@@ -3,7 +3,7 @@
 //
 // The stand-alone stages (ops.cu) cost 13 launches + 2 memsets per scan, each a few microseconds of work on 128k points;
 // here the phases are separated by grid barriers instead of kernel boundaries:
-//   P1 deskew/widen -> frame[], stage-1 claim
+//   P1 deskew/widen -> frame[], stage-1 claim (the IMU variant: limu_deskew_imu's compensation of each record, imu_compensate.cuh)
 //   P2 stage-1 winner flags, per-tile counts, ordered scatter of the winners -> down[], stage-2 claim
 //   P3 (un-claim the stage-1 table) stage-2 winner flags, per-tile counts, ordered scatter -> src0[]
 // Inside P2 / P3 a tile does not wait at a grid barrier for the counts of the tiles before it: every count is published as ONE 8-byte word
@@ -18,6 +18,7 @@
 
 #include "compact.cuh"
 #include "grid_sync.cuh"
+#include "imu_compensate.cuh"
 #include "ops.cuh"
 #include "voxel_map.cuh"
 
@@ -51,6 +52,12 @@ struct VoxelizeArgs {
     unsigned int *barrier;      // [0] grid barrier, [1] exit counter; zero at rest (the last CTA out re-arms them, no memset per launch)
     DevStatus *st;
     DevStatus *st_next;         // non-null: the status word of the NEXT launch of this pipeline (two words alternate); zeroed late in this launch
+};
+// The parameters of the IMU variant (mode 3): a struct of their own, so the parameter block of the other kernels stays as it is.
+// The pose table is read from global memory with ordinary loads, served by L1 (a warp's points mostly share their head row). Not staged in
+// shared memory: the kernel keeps the shared-memory footprint, and so the carve-out, of the plain variants (DESIGN section 4).
+struct VoxelizeImuArgs : VoxelizeArgs {
+    ImuDeskew imu;
 };
 
 // Claim the voxel of p in a scan-local table and note `index` as a candidate for its first point (atomicMin). Each probe is ONE
@@ -126,8 +133,9 @@ __device__ unsigned long long g_vox_marks[8];   // globaltimer of thread 0 of CT
 #define VX_MARK(k) do {} while (0)
 #endif
 
-// VX_BLOCK threads handle tiles of VX_BLOCK consecutive points, one point per thread.
-__device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
+// VX_BLOCK threads handle tiles of VX_BLOCK consecutive points, one point per thread. IMU: the variant of mode 3 (Args = VoxelizeImuArgs).
+template <bool IMU, class Args>
+__device__ __forceinline__ void voxelize_body(const Args &A) {
     __shared__ int ws[32];
     __shared__ int total;
     GridSync gs{A.barrier, 0u, gridDim.x};
@@ -145,7 +153,17 @@ __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
         }
     }
     // P1: frame[i] = deskewed / widened point (icp.cpp:36-47, deskew.cpp:18-26); stage-1 claim at 0.5 v
-    {
+    if constexpr (IMU) {
+        for (int64_t i = gtid; i < n; i += gthreads) {
+            const unsigned char *r = static_cast<const unsigned char *>(A.raw) + (size_t)i * A.stride;
+            const float *q = reinterpret_cast<const float *>(r);
+            float xyz[3] = {q[0], q[1], q[2]};
+            imu_deskew_point(A.imu.table, A.imu.M, i, imu_point_time(r, A.imu.toff), A.imu.rot_end, A.imu.pos_lidar_end, A.imu.p_il, xyz);
+            const V3 p{(double)xyz[0], (double)xyz[1], (double)xyz[2]};   // the float write-back, widened (ekf.cpp:451-468)
+            A.frame[3 * i] = p.x; A.frame[3 * i + 1] = p.y; A.frame[3 * i + 2] = p.z;
+            A.pslot1[i] = claim(A.keys1, A.min1, A.shift1, A.mask1, p, A.vs1, (unsigned int)i, A.st);
+        }
+    } else {
         double tw[6];
         if (A.deskew) {
 #pragma unroll
@@ -241,8 +259,10 @@ __device__ __forceinline__ void voxelize_body(const VoxelizeArgs &A) {
 }
 // The two launch shapes: full (alone on the GPU: 1024 threads x 64 registers = a whole register file) and lean (48 registers, a few
 // spills), which leaves 16 K registers per SM to the map update's CTA that runs beside it in the pipelined odometry path (odometry.cu).
-static __global__ void __launch_bounds__(VX_BLOCK, 1) k_voxelize_full(const VoxelizeArgs A) { voxelize_body(A); }
-static __global__ void __maxnreg__(48) k_voxelize_lean(const VoxelizeArgs A) { voxelize_body(A); }
+static __global__ void __launch_bounds__(VX_BLOCK, 1) k_voxelize_full(const VoxelizeArgs A) { voxelize_body<false>(A); }
+static __global__ void __maxnreg__(48) k_voxelize_lean(const VoxelizeArgs A) { voxelize_body<false>(A); }
+static __global__ void __launch_bounds__(VX_BLOCK, 1) k_voxelize_imu_full(const VoxelizeImuArgs A) { voxelize_body<true>(A); }
+static __global__ void __maxnreg__(48) k_voxelize_imu_lean(const VoxelizeImuArgs A) { voxelize_body<true>(A); }
 
 // One thread that waits until a frame kernel launched EARLIER on another stream has published the pose of its scan (the flag carries that
 // launch's sequence number): the stream it sits in -- the next scan's k_voxelize behind it -- is released the moment the Gauss-Newton loop is
@@ -289,8 +309,9 @@ static int64_t pow2_slots(int64_t n) { int64_t p = 1024; while (p < 2 * n) p <<=
 // Enqueue the fused kernel. raw/ts/twist are device pointers; outputs: frame (n x 3), down, src0, counts[0..1].
 int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int mode, int stride, const double *ts_dev, int deskew, const double *twist_host,
                     int64_t n, double v, double *frame_dev, double *down_dev, double *src0_dev, int *counts_dev, const double *twist_dev, DevStatus *own_status, int *status_used,
-                    cudaStream_t stream, bool beside) {
+                    cudaStream_t stream, bool beside, const ImuDeskew *imu) {
     if (!stream) stream = c->stream;
+    if (mode == 3 && !imu) { set_error("voxelize_device: mode 3 without IMU deskew arguments"); return LIMU_ERR_INVALID; }
     if (n <= 0) {
         LIMU_CUDA_TRY(cudaMemsetAsync(counts_dev, 0, 2 * sizeof(int), stream));
         if (own_status) {   // the word this (empty) launch reports into must read clean; the rotation moves on as for any launch
@@ -337,7 +358,8 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     }
     const int par = sc.parity;
     sc.parity ^= 1;
-    VoxelizeArgs A;
+    VoxelizeImuArgs X;
+    VoxelizeArgs &A = X;
     A.raw = raw_dev; A.ts = ts_dev; A.mode = mode; A.stride = stride; A.deskew = deskew; A.n = n;
     for (int k = 0; k < 6; ++k) A.twist[k] = (deskew && twist_host) ? twist_host[k] : 0.0;
     A.twist_dev = deskew ? twist_dev : nullptr;
@@ -374,7 +396,13 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     // CTA of this cooperative launch has been placed, and this launch sits in front of the loop that gate waits for (see icp_device)
     const int grid = (int)std::min<int64_t>(ntiles, beside ? (int64_t)std::max(1, c->sm_count - GATE_SLACK_SMS) : (int64_t)c->sm_count * g_vx_blocks_per_sm);
     void *args[] = {&A};
-    LIMU_CUDA_TRY(cudaLaunchCooperativeKernel(beside ? (const void *)k_voxelize_lean : (const void *)k_voxelize_full, dim3(grid), dim3(VX_BLOCK), args, 0, stream));
+    const void *fn = beside ? (const void *)k_voxelize_lean : (const void *)k_voxelize_full;
+    if (mode == 3) {
+        X.imu = *imu;
+        args[0] = &X;
+        fn = beside ? (const void *)k_voxelize_imu_lean : (const void *)k_voxelize_imu_full;
+    }
+    LIMU_CUDA_TRY(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(VX_BLOCK), args, 0, stream));
     LIMU_LAUNCHED();
     return LIMU_OK;
 }
