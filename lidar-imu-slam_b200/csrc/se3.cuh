@@ -99,9 +99,17 @@ LIMU_HD void mat3vec(const double *A, const double *v, double *o) {
     o[2] = A[6] * v[0] + (A[7] * v[1] + A[8] * v[2]);
 }
 
+// Correctly rounded 1 / v (on the device without the FP64 division subroutine).
+LIMU_HD double rcp(double v) {
+#ifdef __CUDA_ARCH__
+    return __drcp_rn(v);
+#else
+    return 1.0 / v;
+#endif
+}
+
 // SE3::exp, se3.hpp:852-861; SO3::expAndTheta so3.hpp:694-732; SO3::leftJacobian so3.hpp:550-571.
-// The two halves below (rotation / translation) are independent given the twist; the Gauss-Newton solve evaluates them
-// on two lanes at once. se3_exp() is their composition and is bit-identical to Sophus on x86-64.
+// se3_exp() is the composition of the two halves below and is bit-identical to Sophus on x86-64.
 LIMU_HD void se3_exp_rotation(const double *a, double *q /* x y z w */, double *theta_out) {
     const double *om = a + 3;
     const double theta_sq = sqnorm3(om[0], om[1], om[2]);
@@ -115,7 +123,7 @@ LIMU_HD void se3_exp_rotation(const double *a, double *q /* x y z w */, double *
         theta = sqrt(theta_sq);
         const double half = 0.5 * theta;
 #ifdef __CUDA_ARCH__
-        double sh, ch;   // one argument reduction for both (this sits on the critical path of every Gauss-Newton iteration)
+        double sh, ch;   // one argument reduction for both
         sincos(half, &sh, &ch);
         imag = sh / theta;
         real = ch;
@@ -158,6 +166,38 @@ LIMU_HD Pose se3_exp(const double *a) {
     return Pose{q[0], q[1], q[2], q[3], t[0], t[1], t[2]};
 }
 
+// SE3::exp for the Gauss-Newton loop, where it runs on one thread while the grid waits: the same formulas as se3_exp() from one sqrt
+// and one sincos(theta/2) -- sin(theta) = 2 sh ch, 1 - cos(theta) = 2 sh^2 -- and one reciprocal of theta, and V v as
+// v + c1 (w x v) + c2 (w x (w x v)). Not bit-identical to Sophus: the quaternion differs by rounding, and the translation is the more
+// accurate one where Sophus's 1 - cos(theta) cancels (theta between ~1e-10 and ~1e-5). Nothing keyed or compared bit for bit uses it.
+LIMU_HD Pose se3_exp_gn(const double *a) {
+    const V3 ups{a[0], a[1], a[2]}, om{a[3], a[4], a[5]};
+    const double theta_sq = sqnorm3(om.x, om.y, om.z);
+    const V3 wu = cross(om, ups), wwu = cross(om, wu);
+    double imag, real, c1, c2;
+    if (theta_sq < LIMU_SOPHUS_EPS * LIMU_SOPHUS_EPS) {   // Sophus's small-angle branches: V = I + Omega / 2
+        const double theta_po4 = theta_sq * theta_sq;
+        imag = 0.5 - (1.0 / 48.0) * theta_sq + (1.0 / 3840.0) * theta_po4;
+        real = 1.0 - (1.0 / 8.0) * theta_sq + (1.0 / 384.0) * theta_po4;
+        c1 = 0.5;
+        c2 = 0.0;
+    } else {
+        const double theta = sqrt(theta_sq), it = rcp(theta), half = 0.5 * theta;
+        double sh, ch;
+#ifdef __CUDA_ARCH__
+        sincos(half, &sh, &ch);
+#else
+        sh = sin(half); ch = cos(half);
+#endif
+        imag = sh * it;
+        real = ch;
+        c1 = 2.0 * (imag * imag);                          // (1 - cos theta) / theta^2
+        c2 = (theta - 2.0 * (sh * ch)) * (it * (it * it)); // (theta - sin theta) / theta^3
+    }
+    return Pose{imag * om.x, imag * om.y, imag * om.z, real,
+                (ups.x + c1 * wu.x) + c2 * wwu.x, (ups.y + c1 * wu.y) + c2 * wwu.y, (ups.z + c1 * wu.z) + c2 * wwu.z};
+}
+
 // SE3::log, se3.hpp:237-253; SO3::logAndTheta so3.hpp:264-310; leftJacobianInverse so3.hpp:573-597.
 LIMU_HD void se3_log(const Pose &T, double *x) {
     const double sqn = sqnorm3(T.qx, T.qy, T.qz), w = T.qw;
@@ -196,6 +236,17 @@ LIMU_HD double norm6(const double *x) {
     const double a = (x[0] * x[0] + x[2] * x[2]) + x[4] * x[4];
     const double b = (x[1] * x[1] + x[3] * x[3]) + x[5] * x[5];
     return sqrt(a + b);
+}
+
+// Convergence of a Gauss-Newton iteration, |log(exp(x))| < eps (icp.cpp:124), from the twist itself: log(exp(x)) is x up to rounding
+// while the rotation is below pi, so the verdict is 1 (converged) when |x| < eps (1 - 1e-6) and 0 when |x| > eps (1 + 1e-6). Inside
+// that band, or for |w| >= 3 (or NaN), it is 2: too close to call, and the caller takes the logarithm as the reference does.
+// Compares squares (the band is far wider than their rounding): no sqrt.
+LIMU_HD int gn_verdict(const double *x, double eps) {
+    const double n2 = ((x[0] * x[0] + x[2] * x[2]) + x[4] * x[4]) + ((x[1] * x[1] + x[3] * x[3]) + x[5] * x[5]);   // norm6(x)^2
+    const double lo = eps * (1.0 - 1e-6), hi = eps * (1.0 + 1e-6);
+    if (!(sqnorm3(x[3], x[4], x[5]) < 9.0)) return 2;
+    return n2 < lo * lo ? 1 : (n2 > hi * hi ? 0 : 2);
 }
 
 // Eigen 3.4.0 LDLT<Matrix6d>: diagonal-pivoted in-place factorisation of the lower triangle
@@ -324,6 +375,45 @@ LIMU_HD void expand_normal_equations(const double *S, double *H, double *g) {
     H[4 * 6 + 3] = -xy;     H[4 * 6 + 4] = xx + zz; H[4 * 6 + 5] = -yz;
     H[5 * 6 + 3] = -xz;     H[5 * 6 + 4] = -yz;     H[5 * 6 + 5] = xx + yy;
     g[0] = S[10]; g[1] = S[11]; g[2] = S[12]; g[3] = S[13]; g[4] = S[14]; g[5] = S[15];
+}
+
+// x = H^-1 (-g) straight from the 16 sums, for the point-to-point H above: its top-left block is w I, so eliminating it leaves the 3x3
+// Schur complement Sm = D - A^T A / w = D - (|c|^2 I - c c^T) / w (c = sum w s, D the bottom-right block), solved by its adjugate:
+//   Sm x2 = -g2 + (c x g1) / w,   x1 = (c x x2 - g1) / w.
+// One reciprocal of w, one of det(Sm), no pivot search. Agrees with ldlt6_solve to rounding (the sums are ours, not Eigen's, in any
+// case). When w is not positive and finite, when det(Sm) is not clear of the cancellation in D - A^T A / w (det(Sm) <= 1e-9 tr(D)^3:
+// fewer than three points, collinear points), or when a sum is not finite, it returns exactly what expand_normal_equations +
+// ldlt6_solve return. The choice depends on
+// S alone, so every CTA and rank that folds the same sums takes the same branch.
+LIMU_HD void solve_point_to_point(const double *S, double *x) {
+    const double w = S[0], cx = S[1], cy = S[2], cz = S[3];
+    const double xx = S[4], xy = S[5], xz = S[6], yy = S[7], yz = S[8], zz = S[9];
+    const double iw = rcp(w), mx = cx * iw, my = cy * iw, mz = cz * iw;   // m = c / w
+    const double dxx = yy + zz, dyy = xx + zz, dzz = xx + yy;
+    const double s00 = dxx - (cy * my + cz * mz), s11 = dyy - (cx * mx + cz * mz), s22 = dzz - (cx * mx + cy * my);
+    const double s01 = cx * my - xy, s02 = cx * mz - xz, s12 = cy * mz - yz;
+    const double a00 = s11 * s22 - s12 * s12, a01 = s02 * s12 - s01 * s22, a02 = s01 * s12 - s02 * s11;   // adj(Sm), symmetric
+    const double a11 = s00 * s22 - s02 * s02, a12 = s01 * s02 - s00 * s12, a22 = s00 * s11 - s01 * s01;
+    const double det = (s00 * a00 + s01 * a01) + s02 * a02;
+    const double trd = (dxx + dyy) + dzz, gsum = ((S[10] + S[11]) + (S[12] + S[13])) + (S[14] + S[15]);
+    if (!(w > 0.0 && isfinite(w) && det > 1e-9 * (trd * (trd * trd)) && isfinite(gsum))) {
+        double H[36], g[6];
+        expand_normal_equations(S, H, g);
+#pragma unroll
+        for (int k = 0; k < 6; ++k) g[k] = -g[k];
+        ldlt6_solve(H, g, x);
+        return;
+    }
+    const double g1x = S[10], g1y = S[11], g1z = S[12];
+    const double rx = (my * g1z - mz * g1y) - S[13], ry = (mz * g1x - mx * g1z) - S[14], rz = (mx * g1y - my * g1x) - S[15];
+    const double id = rcp(det);
+    const double x2x = ((a00 * rx + a01 * ry) + a02 * rz) * id;
+    const double x2y = ((a01 * rx + a11 * ry) + a12 * rz) * id;
+    const double x2z = ((a02 * rx + a12 * ry) + a22 * rz) * id;
+    x[0] = (my * x2z - mz * x2y) - g1x * iw;
+    x[1] = (mz * x2x - mx * x2z) - g1y * iw;
+    x[2] = (mx * x2y - my * x2x) - g1z * iw;
+    x[3] = x2x; x[4] = x2y; x[5] = x2z;
 }
 
 }  // namespace limu
