@@ -85,3 +85,49 @@ def np_map_insert(xyz, vox, cap):
     keep = order[rank < cap]
     keys = np_keys(xyz[np.sort(first)], vox).astype(np.int32)
     return keys, np.minimum(sizes, cap).astype(np.int32), xyz[keep]
+
+
+def np_closest(keys, counts, pts, q, vox):
+    """VoxelHashMap::get_closest_neighbour (voxel_hash_map.cpp:64-102) by brute force over a dump (creation order):
+    (a) the query's own voxel exists -> the first minimum of (p - q).squaredNorm() over its stored points, in storage order;
+    (b) else the occupied neighbour of the 27 cells with the largest (|delta|^2, creation position) -- the reference's max-heap
+        top, a later-created voxel wins ties;
+    (c) else (0,0,0). -> (points [n,3], voxel keys [n,3] int32 (INT_MIN where none), ranks [n] int32 (-1 where none))."""
+    q = np.asarray(q, np.float64).reshape(-1, 3)
+    n, nv = len(q), len(keys)
+    packed = np_pack(keys.astype(np.int64))
+    order = np.argsort(packed, kind="stable")
+    spacked = packed[order]
+
+    def find(k):   # creation position of the voxel with key k (rows), -1 where absent
+        p = np_pack(k)
+        i = np.minimum(np.searchsorted(spacked, p), max(nv - 1, 0))
+        return np.where((nv > 0) & (spacked[i] == p), order[i], -1) if nv else np.full(len(k), -1)
+
+    kq = np_keys(q, vox)
+    pos = find(kq)
+    best_d = np.where(pos >= 0, 4, -1)                       # own voxel: beats every neighbour
+    for dx in (-1, 0, 1):
+        for dy in (-1, 0, 1):
+            for dz in (-1, 0, 1):
+                if dx == dy == dz == 0:
+                    continue
+                c = find(kq + np.array([dx, dy, dz]))
+                d = dx * dx + dy * dy + dz * dz
+                better = (c >= 0) & ((d > best_d) | ((d == best_d) & (c > pos)))
+                pos = np.where(better, c, pos)
+                best_d = np.where(better, d, best_d)
+    start = np.r_[0, np.cumsum(counts)].astype(np.int64)
+    out, rank = np.zeros((n, 3)), np.full(n, -1, np.int32)
+    key = np.full((n, 3), np.iinfo(np.int32).min, np.int32)
+    for v in np.unique(pos[pos >= 0]):
+        b = pts[start[v]:start[v + 1]]
+        every = np.flatnonzero(pos == v)
+        step = max(1, 1 << 20 >> max(len(b).bit_length(), 1))
+        for at in range(0, len(every), step):
+            sel = every[at:at + step]
+            dd = q[sel, None, :] - b[None, :, :]
+            d2 = (dd[..., 0] * dd[..., 0] + dd[..., 1] * dd[..., 1]) + dd[..., 2] * dd[..., 2]
+            r = np.argmin(d2, axis=1)                          # first minimum in storage order
+            out[sel], rank[sel], key[sel] = b[r], r, keys[v]
+    return out, key, rank
