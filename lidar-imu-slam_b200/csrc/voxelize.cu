@@ -29,6 +29,9 @@ namespace limu {
 // Threads per CTA and points per tile (one point per thread). One fat CTA per SM: a grid barrier is paid per ARRIVING CTA (atomics on one
 // word serialise at ~4 ns each: 592 CTAs of 256 -> 148 of 1024).
 constexpr int VX_BLOCK = 1024;
+// Deskew transforms one tile keeps in shared memory (one per run of equal timestamps; 3.5 KB). The bench scan has at most 19 runs in a tile;
+// 64 leaves room for sensors with fewer beams per firing (a 16-beam sensor: 64 runs).
+constexpr int VX_RUNS = 64;
 
 struct VoxelizeArgs {
     const void *raw;            // mode 0: float4 {x,y,z,t}; mode 1: records `stride` bytes apart + ts; mode 2: double xyz (already a frame)
@@ -55,7 +58,8 @@ struct VoxelizeArgs {
 };
 // The parameters of the IMU variant (mode 3): a struct of their own, so the parameter block of the other kernels stays as it is.
 // The pose table is read from global memory with ordinary loads, served by L1 (a warp's points mostly share their head row). Not staged in
-// shared memory: the kernel keeps the shared-memory footprint, and so the carve-out, of the plain variants (DESIGN section 4).
+// shared memory: the kernel keeps a small shared-memory footprint (132 B; the plain variants' 4 KB run table included), and so the carve-out
+// next to k_gate (DESIGN section 4).
 struct VoxelizeImuArgs : VoxelizeArgs {
     ImuDeskew imu;
 };
@@ -133,6 +137,15 @@ __device__ unsigned long long g_vox_marks[8];   // globaltimer of thread 0 of CT
 #define VX_MARK(k) do {} while (0)
 #endif
 
+// The motion of a point fired at time t: SE3::exp((t - mid_pose_timestamp) * twist) (deskew.cpp:18-26, deskew.hpp:12).
+__device__ __forceinline__ Pose deskew_motion(double t, const double *tw) {
+    const double s = t - 0.5;
+    double st[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) st[k] = s * tw[k];
+    return se3_exp(st);
+}
+
 // VX_BLOCK threads handle tiles of VX_BLOCK consecutive points, one point per thread. IMU: the variant of mode 3 (Args = VoxelizeImuArgs).
 template <bool IMU, class Args>
 __device__ __forceinline__ void voxelize_body(const Args &A) {
@@ -164,39 +177,65 @@ __device__ __forceinline__ void voxelize_body(const Args &A) {
             A.pslot1[i] = claim(A.keys1, A.min1, A.shift1, A.mask1, p, A.vs1, (unsigned int)i, A.st);
         }
     } else {
-        double tw[6];
-        if (A.deskew) {
+        // the twist in shared memory, not in 12 registers across the loop (k_voxelize_lean has 48)
+        __shared__ double tw[6];
+        if (A.deskew && threadIdx.x == 0) {
 #pragma unroll
-            for (int k = 0; k < 6; ++k) tw[k] = A.twist[k];
-            if (A.twist_dev) {
-#pragma unroll
-                for (int k = 0; k < 6; ++k) tw[k] = __ldcg(A.twist_dev + k);
-            }
+            for (int k = 0; k < 6; ++k) tw[k] = A.twist_dev ? __ldcg(A.twist_dev + k) : A.twist[k];
         }
-        for (int64_t i = gtid; i < n; i += gthreads) {
+        // One tile of VX_BLOCK points per CTA pass (the points the grid-stride loop gave this thread), with a CTA-uniform trip count: the
+        // deskew transform is a function of the timestamp alone, and a spinning LiDAR fires all beams of one azimuth step at the same time
+        // (64 beams per timestamp in the bench scan: ~16 distinct times per tile). So each run of equal timestamps BITS in a tile gets ONE
+        // se3_exp, in a shared table, and every point applies its run's pose: the same operations on the same operands as the per-point
+        // computation, hence bit-identical frames. Equal bits, not equal values: NaN, +-0 and denormals group deterministically. A tile
+        // with more than VX_RUNS runs (per-point times, unsorted clouds) takes the per-point path; the branch is CTA-uniform.
+        __shared__ unsigned long long last_t[VX_BLOCK / 32];   // bits of each warp's last timestamp
+        __shared__ Pose runs[VX_RUNS];                         // the run's timestamp (in .qx) until its pose replaces it
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+            const int64_t i = (int64_t)tile * VX_BLOCK + threadIdx.x;
+            const bool live = i < n;
+            // the timestamp first, the point after its transform is known: p is not live across se3_exp
             double t = 0.0;
-            V3 p;
-            if (A.mode == 0) {
-                const float4 q = __ldg(reinterpret_cast<const float4 *>(A.raw) + i);
-                p = V3{(double)q.x, (double)q.y, (double)q.z};
-                t = (double)q.w;
-            } else if (A.mode == 1) {
-                const float *q = reinterpret_cast<const float *>(static_cast<const unsigned char *>(A.raw) + (size_t)i * A.stride);
-                p = V3{(double)q[0], (double)q[1], (double)q[2]};
-                if (A.deskew) t = A.ts[i];
-            } else {
-                const double *q = static_cast<const double *>(A.raw) + 3 * i;
-                p = V3{q[0], q[1], q[2]};
-            }
+            if (live && A.deskew) t = A.mode == 0 ? (double)__ldg(reinterpret_cast<const float4 *>(A.raw) + i).w : A.mode == 1 ? A.ts[i] : 0.0;
+            Pose T{};
             if (A.deskew) {
-                const double s = t - 0.5;   // mid_pose_timestamp, deskew.hpp:12
-                double st[6];
-#pragma unroll
-                for (int k = 0; k < 6; ++k) st[k] = s * tw[k];
-                p = apply(se3_exp(st), p);
+                const unsigned long long tb = (unsigned long long)__double_as_longlong(t);
+                unsigned long long prev = __shfl_up_sync(0xFFFFFFFFu, tb, 1);
+                if (lane == 31) last_t[warp] = tb;
+                __syncthreads();
+                if (lane == 0 && warp > 0) prev = last_t[warp - 1];
+                const int head = live && (threadIdx.x == 0 || tb != prev);
+                const int run = block_exclusive_scan_count(head, &total, ws) + head - 1;   // (thread 0 of a tile is live: run >= 0 for live points)
+                // one se3_exp site for both branches (two copies of its FP64 state would not fit k_voxelize_lean's 48 registers): with the
+                // table, thread r computes the pose of run r; without it, every point its own
+                const bool table = total <= VX_RUNS;
+                if (table && head) runs[run].qx = t;
+                if (table) __syncthreads();
+                const bool mine = table ? (int)threadIdx.x < total : live;
+                if (mine) T = deskew_motion(table ? runs[threadIdx.x].qx : t, tw);
+                if (table) {
+                    if (mine) runs[threadIdx.x] = T;
+                    __syncthreads();
+                    if (live) T = runs[run];
+                }
             }
-            A.frame[3 * i] = p.x; A.frame[3 * i + 1] = p.y; A.frame[3 * i + 2] = p.z;
-            A.pslot1[i] = claim(A.keys1, A.min1, A.shift1, A.mask1, p, A.vs1, (unsigned int)i, A.st);
+            if (live) {
+                V3 p;
+                if (A.mode == 0) {
+                    const float4 q = __ldg(reinterpret_cast<const float4 *>(A.raw) + i);
+                    p = V3{(double)q.x, (double)q.y, (double)q.z};
+                } else if (A.mode == 1) {
+                    const float *q = reinterpret_cast<const float *>(static_cast<const unsigned char *>(A.raw) + (size_t)i * A.stride);
+                    p = V3{(double)q[0], (double)q[1], (double)q[2]};
+                } else {
+                    const double *q = static_cast<const double *>(A.raw) + 3 * i;
+                    p = V3{q[0], q[1], q[2]};
+                }
+                if (A.deskew) p = apply(T, p);
+                A.frame[3 * i] = p.x; A.frame[3 * i + 1] = p.y; A.frame[3 * i + 2] = p.z;
+                A.pslot1[i] = claim(A.keys1, A.min1, A.shift1, A.mask1, p, A.vs1, (unsigned int)i, A.st);
+            }
         }
     }
     gs.sync();
