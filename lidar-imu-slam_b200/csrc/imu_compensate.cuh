@@ -14,6 +14,14 @@ namespace limu {
 
 constexpr int IMU_MAX_ROWS = 96;   // table rows (kalman::Pose6D, 22 doubles each) a call accepts
 
+// The IMU deskew arguments of one limu_odom_register_cloud_imu / limu_odom_prefetch_cloud_imu call, copied from the caller (host): a prepared
+// scan is only used by a call whose arguments are byte for byte the same.
+struct ImuCall {
+    int32_t M, toff;
+    double rot_end[9], pos_lidar_end[3], p_il[3];
+    double table[IMU_MAX_ROWS * 22];
+};
+
 // Eigen::AngleAxisd(dt*|w|, w.normalized()).toRotationMatrix() (Eigen/src/Geometry/AngleAxis.h)
 __device__ __forceinline__ void ang_vel_to_rmat(const double *w, double dt, double *R) {
     const double z = sqnorm3(w[0], w[1], w[2]);

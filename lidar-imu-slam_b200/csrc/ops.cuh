@@ -33,18 +33,33 @@ struct ImuDeskew {
     int M, toff;
     double rot_end[9], pos_lidar_end[3], p_il[3];
 };
-// KissICP::deskew_scan + the two voxel_downsample stages of KissICP::voxelize in one cooperative launch.
-// mode 0: raw = float4 {x,y,z,t}; 1: records `stride` bytes apart + FP64 ts; 2: double xyz (register_frame(Vec3dVector));
-// 3: records `stride` bytes apart, IMU-deskewed as limu_deskew_imu does (`imu`; deskew / twist are not read).
-// twist_dev (speculative launches, odometry.cu): read the deskew twist from device memory instead of twist_host.
+struct ImuCall;   // the arguments of one IMU-deskewing call (imu_compensate.cuh)
+// One scan in device memory as k_voxelize reads it.
+enum ScanLayout {
+    SCAN_XYZT = 0,      // float4 {x,y,z,t}
+    SCAN_RECORDS = 1,   // records `stride` bytes apart (float x,y,z first) + FP64 timestamps `ts`
+    SCAN_XYZ = 2,       // double xyz (register_frame(Vec3dVector)): already a frame, never deskewed
+    SCAN_IMU = 3,       // records `stride` bytes apart, IMU-deskewed as limu_deskew_imu does with `imu` and the pose table at `imu_table`
+};
+struct Scan {
+    int layout = SCAN_XYZT;
+    const void *ptr = nullptr;
+    int stride = 0;
+    const double *ts = nullptr;
+    const ImuCall *imu = nullptr;
+    const double *imu_table = nullptr;
+    int64_t n = 0;
+};
+// KissICP::deskew_scan + the two voxel_downsample stages of KissICP::voxelize in one cooperative launch. deskew (layouts 0 and 1): with the
+// twist at twist_host, or at twist_dev (device memory: speculative launches, odometry.cu).
 // own_status: THREE status words private to the pipeline that owns `sc` (zero at first use): consecutive launches rotate through them and each
 // launch zeroes the next one late, so a word is clean when its launch starts without a memset per scan; *status_used = which word this launch
 // reports into. nullptr = the context's shared word.
-// stream: where to enqueue (nullptr = the context's); beside: half-size CTAs, one per SM, so that the launch fits next to another kernel's CTA.
-int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int mode, int stride, const double *ts_dev, int deskew, const double *twist_host,
-                    int64_t n, double v, double *frame_dev, double *down_dev, double *src0_dev, int *counts_dev, const double *twist_dev = nullptr,
-                    DevStatus *own_status = nullptr, int *status_used = nullptr, cudaStream_t stream = nullptr, bool beside = false,
-                    const ImuDeskew *imu = nullptr);
+// stream: where to enqueue (nullptr = the context's); beside: the lean kernel on all but GATE_SLACK_SMS SMs, so that the launch runs next to the
+// map update of the pipelined path.
+int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const Scan &scan, int deskew, const double *twist_host, double v, double *frame_dev, double *down_dev,
+                    double *src0_dev, int *counts_dev, const double *twist_dev = nullptr, DevStatus *own_status = nullptr, int *status_used = nullptr,
+                    cudaStream_t stream = nullptr, bool beside = false);
 // One-thread kernel on stream s that returns once *flag has reached seq (voxelize.cu).
 int gate_device(cudaStream_t s, const unsigned int *flag, unsigned int seq);
 

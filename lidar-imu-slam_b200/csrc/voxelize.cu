@@ -345,12 +345,12 @@ static int g_vx_blocks_per_sm = 0;
 
 static int64_t pow2_slots(int64_t n) { int64_t p = 1024; while (p < 2 * n) p <<= 1; return p; }
 
-// Enqueue the fused kernel. raw/ts/twist are device pointers; outputs: frame (n x 3), down, src0, counts[0..1].
-int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int mode, int stride, const double *ts_dev, int deskew, const double *twist_host,
-                    int64_t n, double v, double *frame_dev, double *down_dev, double *src0_dev, int *counts_dev, const double *twist_dev, DevStatus *own_status, int *status_used,
-                    cudaStream_t stream, bool beside, const ImuDeskew *imu) {
+// Enqueue the fused kernel. outputs: frame (n x 3), down, src0, counts[0..1].
+int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const Scan &scan, int deskew, const double *twist_host, double v, double *frame_dev, double *down_dev,
+                    double *src0_dev, int *counts_dev, const double *twist_dev, DevStatus *own_status, int *status_used, cudaStream_t stream, bool beside) {
     if (!stream) stream = c->stream;
-    if (mode == 3 && !imu) { set_error("voxelize_device: mode 3 without IMU deskew arguments"); return LIMU_ERR_INVALID; }
+    if (scan.layout == SCAN_IMU && !scan.imu) { set_error("voxelize_device: an IMU scan without IMU deskew arguments"); return LIMU_ERR_INVALID; }
+    const int64_t n = scan.n;
     if (n <= 0) {
         LIMU_CUDA_TRY(cudaMemsetAsync(counts_dev, 0, 2 * sizeof(int), stream));
         if (own_status) {   // the word this (empty) launch reports into must read clean; the rotation moves on as for any launch
@@ -399,7 +399,7 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     sc.parity ^= 1;
     VoxelizeImuArgs X;
     VoxelizeArgs &A = X;
-    A.raw = raw_dev; A.ts = ts_dev; A.mode = mode; A.stride = stride; A.deskew = deskew; A.n = n;
+    A.raw = scan.ptr; A.ts = scan.ts; A.mode = scan.layout; A.stride = scan.stride; A.deskew = deskew; A.n = n;
     for (int k = 0; k < 6; ++k) A.twist[k] = (deskew && twist_host) ? twist_host[k] : 0.0;
     A.twist_dev = deskew ? twist_dev : nullptr;
     A.vs1 = v * 0.5; A.vs2 = v * 1.5;
@@ -436,8 +436,10 @@ int voxelize_device(limu_ctx *c, VoxelizeScratch &sc, const void *raw_dev, int m
     const int grid = (int)std::min<int64_t>(ntiles, beside ? (int64_t)std::max(1, c->sm_count - GATE_SLACK_SMS) : (int64_t)c->sm_count * g_vx_blocks_per_sm);
     void *args[] = {&A};
     const void *fn = beside ? (const void *)k_voxelize_lean : (const void *)k_voxelize_full;
-    if (mode == 3) {
-        X.imu = *imu;
+    if (scan.layout == SCAN_IMU) {
+        const ImuCall &a = *scan.imu;
+        X.imu.table = scan.imu_table; X.imu.M = a.M; X.imu.toff = a.toff;
+        memcpy(X.imu.rot_end, a.rot_end, sizeof a.rot_end); memcpy(X.imu.pos_lidar_end, a.pos_lidar_end, sizeof a.pos_lidar_end); memcpy(X.imu.p_il, a.p_il, sizeof a.p_il);
         args[0] = &X;
         fn = beside ? (const void *)k_voxelize_imu_lean : (const void *)k_voxelize_imu_full;
     }
