@@ -174,6 +174,23 @@ enum { LIMU_ICP_REFERENCE = 0, LIMU_ICP_NN27 = 1, LIMU_ICP_PLANE = 2 };
 int limu_icp_ex(limu_map *m, const double *xyz, int64_t n, const double init_guess[7], double max_corresp_dist, double kernel,
                 int icp_max_iteration, double est_threshold, int32_t icp_mode, double pose_out[7], limu_icp_stats *stats,
                 double *est_trace, int64_t *ncorr_trace, double *hg_trace);
+/* lidar::ICP (registration.cpp:94-130) from k initial guesses at once (no counterpart in the reference): relocalization against an
+ * existing map from a grid of coarse poses. Every hypothesis is an independent Gauss-Newton loop with limu_icp_ex's semantics
+ * (empty map or icp_max_iteration <= 0: the guess with 0 iterations; a non-finite guess affects only its own result), and its result
+ * does not depend on k or on its position in the list. After its loop, one more correspondence pass over the final working cloud
+ * (the source points moved by every estimate, as the reference leaves them) under the same neighbour rule and max_corresp_dist test
+ * gives `inliers` and rms = sqrt(sum d^2 / inliers) (0 without inliers). init_guesses / poses_out: 7 k doubles; out (optional): k
+ * records; best (optional): the index with the most inliers, then the smaller rms, then the lower index (-1 when k == 0).
+ * icp_mode: LIMU_ICP_REFERENCE or LIMU_ICP_NN27 (LIMU_ICP_PLANE: LIMU_ERR_INVALID). Device scratch grows with the hypotheses that run
+ * at the same time (a working cloud of 24 n bytes each), not with k. On a map of an odometry handle (limu_odom_map) the call is
+ * ordered like limu_icp: it only reads the map. */
+typedef struct limu_icp_hypothesis {
+    int32_t iterations, converged;
+    int64_t inliers;
+    double rms;
+} limu_icp_hypothesis;
+int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init_guesses, int32_t k, double max_corresp_dist, double kernel,
+                   int icp_max_iteration, double est_threshold, int32_t icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best);
 /* get_closest_neighbour under a neighbour rule (icp_mode as above); outputs as limu_map_closest. */
 int limu_map_closest_ex(limu_map *m, const double *xyz, int64_t n, int32_t icp_mode, double *out_xyz, int32_t *out_key, int32_t *out_rank);
 

@@ -32,5 +32,32 @@ namespace lidar
                                     max_corresp_dist, kernel, icp_max_iteration, est_threshold, pose, nullptr, nullptr, nullptr, nullptr), "ICP");
         return limu_dropin::from_pose7(pose);
     }
+
+    // lidar::ICP from every guess of init_guesses in one launch (limu_icp_multi; no counterpart in the reference): relocalization against
+    // an existing map. Returns the pose each guess converged to and its record (iterations, converged, inliers, rms); best_index (optional)
+    // receives the hypothesis with the most inliers, then the smaller rms, then the lower index (-1 without guesses).
+    struct ICPMultiResult
+    {
+        std::vector<SE3d> poses;
+        std::vector<limu_icp_hypothesis> hypotheses;
+        int best = -1;
+    };
+    inline ICPMultiResult ICP_multi(VoxelHashMap &local_map, const utils::Vec3dVector &points, const std::vector<SE3d> &init_guesses,
+                                    const double max_corresp_dist, const double kernel, const int &icp_max_iteration, const double &est_threshold)
+    {
+        const size_t k = init_guesses.size();
+        std::vector<double> init(7 * k), poses(7 * k);
+        for (size_t i = 0; i < k; ++i) limu_dropin::to_pose7(init_guesses[i], init.data() + 7 * i);
+        ICPMultiResult r;
+        r.hypotheses.resize(k);
+        int32_t best = -1;
+        limu_dropin::check(limu_icp_multi(local_map.handle(), points.empty() ? nullptr : points.front().data(), static_cast<int64_t>(points.size()),
+                                          init.data(), static_cast<int32_t>(k), max_corresp_dist, kernel, icp_max_iteration, est_threshold,
+                                          LIMU_ICP_REFERENCE, poses.data(), r.hypotheses.data(), &best), "ICP_multi");
+        r.poses.reserve(k);
+        for (size_t i = 0; i < k; ++i) r.poses.push_back(limu_dropin::from_pose7(poses.data() + 7 * i));
+        r.best = best;
+        return r;
+    }
 }
 #endif

@@ -41,6 +41,10 @@ class IcpStats(C.Structure):
                 ("mean_candidates", C.c_double), ("miss_fraction", C.c_double)]
 
 
+class IcpHypothesis(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("converged", C.c_int32), ("inliers", C.c_int64), ("rms", C.c_double)]
+
+
 class OdomConfig(C.Structure):
     _fields_ = [("voxel_size", C.c_double), ("max_range", C.c_double), ("max_points_per_voxel", C.c_int32),
                 ("deskew", C.c_int32), ("min_motion_th", C.c_double), ("icp_max_iteration", C.c_int32),
@@ -172,6 +176,8 @@ def lib():
             "limu_map_dump": [_vp, _ip, _ip, _dp, C.c_int64, C.c_int64, _lp, _lp],
             "limu_icp": [_vp, _dp, C.c_int64, _dp, C.c_double, C.c_double, C.c_int, C.c_double, _dp, C.POINTER(IcpStats), _dp, _lp, _dp],
             "limu_icp_ex": [_vp, _dp, C.c_int64, _dp, C.c_double, C.c_double, C.c_int, C.c_double, C.c_int32, _dp, C.POINTER(IcpStats), _dp, _lp, _dp],
+            "limu_icp_multi": [_vp, _dp, C.c_int64, _dp, C.c_int32, C.c_double, C.c_double, C.c_int, C.c_double, C.c_int32, _dp, C.POINTER(IcpHypothesis),
+                               C.POINTER(C.c_int32)],
             "limu_map_closest_ex": [_vp, _dp, C.c_int64, C.c_int32, _dp, _ip, _ip],
             "limu_icp_dev": [_vp, _vp, C.c_int64, _dp, C.c_double, C.c_double, C.c_int, C.c_double, _dp, C.POINTER(IcpStats)],
             "limu_comm_create": [_vp, C.c_int, C.c_int, C.c_char_p], "limu_comm_connect": [_vp, C.c_char_p], "limu_comm_destroy": [_vp],
@@ -549,6 +555,22 @@ class VoxelHashMap:
         if trace:
             r.update(est=est[: st.iterations], ncorr=nc[: st.iterations], hg=hg[: st.iterations])
         return r
+
+    def icp_multi(self, xyz, guesses, max_corresp_dist, kernel, icp_max_iteration, est_threshold, icp_mode=0):
+        """lidar::ICP from every row of guesses [k, 7] in one launch (limu_icp_multi): relocalization against this map.
+        Returns dict(poses [k,7], iters [k], converged [k], inliers [k], rms [k], best); best = most inliers, then smaller rms, then lower index."""
+        xyz = _pts(xyz)
+        g = np.ascontiguousarray(np.asarray(guesses, np.float64).reshape(-1, 7))
+        k = len(g)
+        poses = np.empty((max(k, 1), 7))
+        hyp = (IcpHypothesis * max(k, 1))()
+        best = C.c_int32(-1)
+        _chk(lib().limu_icp_multi(self.h, _d(xyz), len(xyz), _d(g), k, float(max_corresp_dist), float(kernel), int(icp_max_iteration),
+                                  float(est_threshold), int(icp_mode), _d(poses), hyp, C.byref(best)))
+        return {"poses": poses[:k].copy(), "iters": np.array([hyp[i].iterations for i in range(k)], np.int32),
+                "converged": np.array([bool(hyp[i].converged) for i in range(k)], bool),
+                "inliers": np.array([hyp[i].inliers for i in range(k)], np.int64), "rms": np.array([hyp[i].rms for i in range(k)]),
+                "best": best.value}
 
     def icp_dev(self, xyz_dev_ptr, n, init_guess, max_corresp_dist, kernel, icp_max_iteration, est_threshold):
         pose = np.empty(7)

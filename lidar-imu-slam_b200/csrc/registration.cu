@@ -1152,6 +1152,213 @@ int icp_device(limu_map *m, IcpArgs A, int64_t n_hint, int icp_mode, bool sharde
     return LIMU_OK;
 }
 
+// ---- multi-hypothesis registration: K Gauss-Newton loops of the latency shape in one launch --------------------------------------------
+// Relocalization runs ICP of one scan against one map from a grid of initial guesses and keeps the best. One loop of the latency shape
+// leaves most of the GPU idle (a few thousand keypoints on ~72 CTAs), so here every hypothesis is run by a GROUP of G CTAs with the
+// loop's own device functions (query pass and memo, LDLT / Schur solve, se3_exp_gn, gn_verdict, stamped row exchange), and a persistent
+// cooperative grid of as many groups as are co-resident takes the hypotheses in waves (group g serves hypotheses g, g + groups, ...).
+// G depends on the query count only, so a hypothesis's sums -- and its result -- do not depend on K or on its place in the list.
+constexpr int MULTI_STEPS = 16;        // query steps of a warp per pass that G aims at (G = ceil(8 n / (224 MULTI_STEPS)), 1 ... 8)
+constexpr int MULTI_OUT = 12;          // doubles per hypothesis: pose 7, iterations, converged, inliers, sum of d^2, pad
+constexpr int MULTI_MAX_G = ICP_BLOCK / 32;   // one row per warp in the fold below
+
+int icp_multi_group_ctas(int64_t n) {
+    return (int)std::min<int64_t>(MULTI_MAX_G, std::max<int64_t>(1, div_up(std::max<int64_t>(n, 1) * 8, (int64_t)(ICP_BLOCK - 32) * MULTI_STEPS)));
+}
+
+struct MultiArgs {
+    IcpArgs A;                 // map, points, tau_sq, th, max_iter, eps, partials, ll_stamp_base, map_counters; work = groups x n x 3
+    const double *guesses;     // k x 7
+    double *out;               // k x MULTI_OUT
+    int k, group_ctas;
+};
+
+// Fitness of a converged hypothesis: correspondences of its final working cloud under the loop's neighbour rule and tau^2 test, counted and
+// their squared distances summed by the group's leading lane (transform: the cloud still needs the last estimate applied).
+template <bool NN27, int ROUNDS>
+__device__ __forceinline__ void fitness_pass_grouped(const IcpArgs &A, const volatile double *Pv, const double *in, bool transform, int64_t n, int64_t gbase,
+                                                     int64_t gstride, int lane, int &inliers, double &d2sum) {
+    const int l8 = lane & 7;
+    const unsigned gmask = 0xFFu << (lane & 24);
+    for (int64_t q0 = gbase - (lane >> 3); q0 < n; q0 += gstride) {
+        const int64_t q = q0 + (lane >> 3);
+        if (q >= n) continue;   // group-uniform
+        const Pose P{Pv[0], Pv[1], Pv[2], Pv[3], Pv[4], Pv[5], Pv[6]};
+        const V3 raw{in[3 * q], in[3 * q + 1], in[3 * q + 2]};
+        const V3 s = transform ? apply(P, raw) : raw;
+        V3 tg{0.0, 0.0, 0.0};
+        int slot = -1, count = 0, own = 1, rank = -1;
+        double d2 = 0.0;
+        if (NN27) group8_closest27(A.map, s, gmask, l8, slot, count, own, d2, rank);
+        else group8_closest<ROUNDS>(A.map, s, gmask, l8, slot, count, own, d2, rank, tg);
+        if (rank < 0) d2 = sqnorm3(s.x, s.y, s.z);   // nothing found -> (0,0,0), range-tested like a real point
+        if (l8 == 0 && d2 < A.tau_sq) { ++inliers; d2sum += d2; }
+    }
+}
+
+// Publish this CTA's row (thread t < NS holds column t as `mine`) with the exchange's stamp, then fold the G rows of the group: warp g
+// reads row g, thread t adds the eight warp values in warp order -- the order of the loop kernel's fold for a grid of G <= 8 CTAs.
+__device__ __forceinline__ void multi_exchange(unsigned long long *rows, int G, int rank, unsigned int stamp, double mine, double *red, double *S) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x < NS) ll_store(rows + ((size_t)rank * NS + threadIdx.x) * 2, mine, stamp);
+    double v = 0.0;
+    if (warp < G && lane < NS) {
+        unsigned int spins = 0u;
+        while (!ll_load(rows + ((size_t)warp * NS + lane) * 2, stamp, v))
+            if (++spins > (1u << 24)) __trap();   // a CTA of the group never published its row: fail loudly instead of hanging the device
+    }
+    __syncthreads();   // (every reader of red is done)
+    red[warp * 32 + lane] = 0.0 + v;
+    __syncthreads();
+    if (threadIdx.x < NS) {
+        double s = 0.0;
+#pragma unroll
+        for (int w = 0; w < ICP_BLOCK / 32; ++w) s += red[w * 32 + threadIdx.x];
+        S[threadIdx.x] = s;
+    }
+    __syncthreads();
+}
+
+template <bool NN27>
+static __global__ void __launch_bounds__(ICP_BLOCK, 2) k_icp_multi(const MultiArgs M) {
+    constexpr int QW = ICP_BLOCK / 32 - 1;   // query warps; the last warp is the solver warp, as in k_icp_persistent
+    __shared__ double red[(ICP_BLOCK / 32) * 32];
+    __shared__ double S[NS];
+    __shared__ double E[7], Tinit[7], Ticp[7];
+    __shared__ int done, verdict;
+    const int G = M.group_ctas, grp = (int)blockIdx.x / G, rank = (int)blockIdx.x % G, groups = (int)gridDim.x / G;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t n = M.A.n_max;
+    IcpArgs A = M.A;
+    A.work = M.A.work + (size_t)grp * 3 * (size_t)n;   // this group's working cloud
+    unsigned long long *rows0 = reinterpret_cast<unsigned long long *>(A.partials) + (size_t)grp * 2 * G * NS * 2;   // two parities of G rows
+    const int64_t gbase = (((int64_t)rank * QW + warp) * 32) / 8 + (lane >> 3), gstride = (int64_t)G * QW * 4;
+    const bool run_icp = !(__ldcg(A.map_counters) == 0ull || A.max_iter <= 0);   // ICP :99-100: empty map -> init_guess
+    unsigned int x = 0u;   // exchanges this group made so far: its stamps never repeat across the hypotheses it serves
+    QueryMemo memo;        // (keyed by voxel index: the map does not change inside the launch, so it stays valid from one hypothesis to the next)
+    memo.own = -1; memo.kx = memo.ky = memo.kz = 0; memo.slot = -1; memo.count = 0;
+    for (int h = grp; h < M.k; h += groups) {
+        __syncthreads();   // the previous hypothesis is finished with the shared state
+        if (threadIdx.x < 7) { Tinit[threadIdx.x] = M.guesses[7 * (size_t)h + threadIdx.x]; Ticp[threadIdx.x] = threadIdx.x == 3 ? 1.0 : 0.0; }
+        if (threadIdx.x < NS) S[threadIdx.x] = 0.0;
+        if (threadIdx.x == 0) { verdict = 0; done = 0; }
+        __syncthreads();
+        int j = 0, converged = 0;
+        bool fresh = false;   // the working cloud already holds the final estimate applied (a pass was made after the converging iteration)
+        if (run_icp) for (;;) {
+            const bool no_more = j >= A.max_iter;
+            if (warp < QW) {
+                if (!no_more) {
+                    double acc = 0.0;
+                    int ncorr = 0, ncand = 0, nmiss = 0;   // (statistics of the single loop; not reported per hypothesis)
+                    const volatile double *Pv = j == 0 ? Tinit : E;
+                    const double *in = j == 0 ? A.points : A.work;
+                    if (A.map.cap <= 8) icp_query_pass_grouped<NN27, false, 1>(A, Pv, in, nullptr, n, gbase, gstride, lane, acc, ncorr, ncand, nmiss, &memo, nullptr);
+                    else if (A.map.cap <= 16) icp_query_pass_grouped<NN27, false, 2>(A, Pv, in, nullptr, n, gbase, gstride, lane, acc, ncorr, ncand, nmiss, &memo, nullptr);
+                    else icp_query_pass_grouped<NN27, false, 3>(A, Pv, in, nullptr, n, gbase, gstride, lane, acc, ncorr, ncand, nmiss, &memo, nullptr);
+                    red[warp * 32 + lane] = (lane & 1) ? 0.0 : acc;   // lane 2i holds sum i
+                }
+            } else if (j > 0) {
+                // tail of iteration j-1, overlapped with pass j: T_icp = estimate * T_icp (:122), |log(estimate)| < eps (:124) when the twist left it open
+                const Pose est = pose_load(E);
+                if (lane == 0) pose_store(mul(est, pose_load(Ticp)), Ticp);
+                if (lane == 1 && verdict == 2) {
+                    double lg[6];
+                    se3_log(est, lg);
+                    done = norm6(lg) < A.eps;
+                }
+            }
+            __syncthreads();
+            if (j > 0 && verdict == 2 && done) { converged = 1; fresh = !no_more; break; }
+            if (no_more) break;
+            double mine = 0.0;
+            if (threadIdx.x < NS) {   // the CTA row in the loop kernel's layout: 16 sums from the even lanes (the counters stay zero)
+                const int src_lane = threadIdx.x < 16 ? 2 * (int)threadIdx.x : 2 * ((int)threadIdx.x - 16) + 1;
+#pragma unroll
+                for (int w = 0; w < QW; ++w) mine += red[w * 32 + src_lane];
+            }
+            const unsigned int stamp = 0x80000000u | ((A.ll_stamp_base + x) & 0x7FFFFFFFu);
+            multi_exchange(rows0 + (size_t)(x & 1u) * G * NS * 2, G, rank, stamp, mine, red, S);
+            ++x;
+            if (warp == QW && lane == 0) {
+                double xv[6];
+                solve_point_to_point(S, xv);
+                pose_store(se3_exp_gn(xv), E);
+                verdict = gn_verdict(xv, A.eps);
+            }
+            __syncthreads();
+            ++j;
+            if (verdict == 1) {
+                if (warp == QW && lane == 0) pose_store(mul(pose_load(E), pose_load(Ticp)), Ticp);
+                converged = 1;
+                __syncthreads();
+                break;
+            }
+        }
+        // fitness over src_after: points * init_guess when the loop did not run, else the working cloud (plus the last estimate unless applied)
+        int inliers = 0;
+        double d2sum = 0.0;
+        if (warp < QW) {
+            const volatile double *Pv = run_icp ? E : Tinit;
+            const double *in = run_icp ? A.work : A.points;
+            if (NN27 || A.map.cap <= 8) fitness_pass_grouped<NN27, 1>(A, Pv, in, !fresh, n, gbase, gstride, lane, inliers, d2sum);
+            else if (A.map.cap <= 16) fitness_pass_grouped<NN27, 2>(A, Pv, in, !fresh, n, gbase, gstride, lane, inliers, d2sum);
+            else fitness_pass_grouped<NN27, 3>(A, Pv, in, !fresh, n, gbase, gstride, lane, inliers, d2sum);
+            inliers = __reduce_add_sync(0xFFFFFFFFu, inliers);
+            d2sum = warp_sum(d2sum);
+        }
+        if (lane == 0) { red[warp * 32] = (double)inliers; red[warp * 32 + 1] = d2sum; }
+        __syncthreads();
+        double mine = 0.0;
+        if (threadIdx.x < 2) {
+#pragma unroll
+            for (int w = 0; w < QW; ++w) mine += red[w * 32 + threadIdx.x];
+        }
+        const unsigned int stamp = 0x80000000u | ((A.ll_stamp_base + x) & 0x7FFFFFFFu);
+        multi_exchange(rows0 + (size_t)(x & 1u) * G * NS * 2, G, rank, stamp, mine, red, S);
+        ++x;
+        if (rank == 0 && threadIdx.x == 0) {
+            double *o = M.out + (size_t)h * MULTI_OUT;
+            pose_store(run_icp ? mul(pose_load(Ticp), pose_load(Tinit)) : pose_load(Tinit), o);   // new_pose = T_icp * init_guess (:129)
+            o[7] = (double)j; o[8] = (double)converged; o[9] = S[0]; o[10] = S[1];
+        }
+    }
+}
+
+// Fitness of one hypothesis of the bandwidth shape (the loop kernel run once per guess): src_after is rebuilt from the points by the guess
+// and the estimates of the loop's iterations applied in turn, as the loop applied them; one thread per query; block rows folded on the host.
+template <bool NN27>
+static __global__ void __launch_bounds__(ICP_BLOCK) k_icp_fitness(const MapView map, const double *points, int64_t n, const double *poses, int nposes,
+                                                                   double tau_sq, double *rows /* [grid][2]: inliers, sum of d^2 */) {
+    __shared__ double red[2][ICP_BLOCK / 32];
+    double inliers = 0.0, d2sum = 0.0;
+    for (int64_t q = (int64_t)blockIdx.x * ICP_BLOCK + threadIdx.x; q < n; q += (int64_t)gridDim.x * ICP_BLOCK) {
+        V3 s{points[3 * q], points[3 * q + 1], points[3 * q + 2]};
+        for (int p = 0; p < nposes; ++p) s = apply(pose_load(poses + 7 * p), s);
+        Nearest nn;
+        nn.rank = -1;
+        if (NN27) {
+            nn = map_closest27(map, s);
+        } else {
+            int count = 0, own = 1;
+            const int slot = map_locate(map, s, &count, &own);
+            if (slot >= 0) block_closest(map, slot, count, s, nn);
+        }
+        const double d2 = nn.rank >= 0 ? sqnorm3(nn.x - s.x, nn.y - s.y, nn.z - s.z) : sqnorm3(s.x, s.y, s.z);
+        if (d2 < tau_sq) { inliers += 1.0; d2sum += d2; }
+    }
+    inliers = warp_sum(inliers);   // fixed trees: warp, then warps in order
+    d2sum = warp_sum(d2sum);
+    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = inliers; red[1][threadIdx.x >> 5] = d2sum; }
+    __syncthreads();
+    if (threadIdx.x < 2) {
+        double v = 0.0;
+#pragma unroll
+        for (int w = 0; w < ICP_BLOCK / 32; ++w) v += red[threadIdx.x][w];
+        rows[2 * (size_t)blockIdx.x + threadIdx.x] = v;
+    }
+}
+
 #ifdef LIMU_ICP_PHASE_TIMING
 extern "C" int limu_debug_frame_marks(double out[72]) {
     unsigned long long h[72];
@@ -1302,7 +1509,97 @@ static int icp_common(limu_map *m, const double *points_dev, int64_t n, const do
     return check_status(c);
 }
 
+// All k hypotheses of the latency shape in one cooperative launch; res: k x MULTI_OUT doubles (host).
+static int icp_multi_grouped(limu_map *m, int64_t n, const double *guesses, int k, double tau, double th, int max_iter, double eps, bool nn27, double *res) {
+    limu_ctx *c = m->ctx;
+    const int G = icp_multi_group_ctas(n);
+    const void *fn = nn27 ? (const void *)k_icp_multi<true> : (const void *)k_icp_multi<false>;
+    int per_sm = 0;
+    LIMU_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, ICP_BLOCK, 0));
+    // every CTA spins on the rows of its group, so the whole grid must be co-resident -- with GATE_SLACK_SMS SMs left for the k_gate threads
+    // of a pipelined odometry handle that may sit on the GPU when this grid is placed (DESIGN section 4, "A launch that needs every SM")
+    const int resident = std::min(std::max(per_sm, 1) * std::max(1, c->sm_count - GATE_SLACK_SMS), icp_partial_rows(c));
+    const int groups = std::max(1, std::min(k, resident / G));
+    LIMU_TRY(c->tmp4.reserve((size_t)groups * (size_t)std::max<int64_t>(n, 1) * 24, c->stream));   // one working cloud per running group
+    LIMU_TRY(icp_partials_reserve(c, c->ll_rows, c->stream));
+    LIMU_TRY(stage_in(c, c->tmp5, guesses, (size_t)k * 7 * sizeof(double)));
+    LIMU_TRY(c->tmp3.reserve((size_t)k * MULTI_OUT * sizeof(double), c->stream));
+    MultiArgs M;
+    memset(&M, 0, sizeof M);
+    IcpArgs &A = M.A;
+    A.map = m->view(); A.map_counters = m->counters.as<unsigned long long>();
+    A.points = c->in0.as<double>(); A.work = c->tmp4.as<double>(); A.n_max = n;
+    A.tau_sq = tau * tau; A.th = th; A.max_iter = max_iter; A.eps = eps;
+    A.partials = c->ll_rows.as<double>();
+    A.ll_stamp_base = c->ll_seq;
+    const unsigned int waves = (unsigned int)div_up(k, groups);   // a group makes at most max_iter + 1 exchanges per hypothesis (the last: its fitness)
+    c->ll_seq = (c->ll_seq + waves * ((unsigned int)std::max(max_iter, 0) + 1u) + 2u) & 0x7FFFFFFFu;
+    M.guesses = c->tmp5.as<double>(); M.out = c->tmp3.as<double>(); M.k = k; M.group_ctas = G;
+    void *args[] = {&M};
+    LIMU_CUDA_TRY(cudaLaunchCooperativeKernel(fn, dim3(groups * G), dim3(ICP_BLOCK), args, 0, c->stream));
+    LIMU_LAUNCHED();
+    LIMU_CUDA_TRY(cudaMemcpyAsync(res, M.out, (size_t)k * MULTI_OUT * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    return check_status(c);
+}
+
+// One hypothesis outside the latency shape: the loop kernel itself (its estimates traced), then the fitness of src_after.
+static int icp_multi_single(limu_map *m, int64_t n, const double guess[7], double tau, double th, int max_iter, double eps, int icp_mode, double *res) {
+    limu_ctx *c = m->ctx;
+    std::vector<double> poses(7 * ((size_t)std::max(max_iter, 1) + 1));
+    std::copy(guess, guess + 7, poses.begin());
+    limu_icp_stats st;
+    LIMU_TRY(icp_common(m, c->in0.as<double>(), n, guess, tau, th, max_iter, eps, res, &st, poses.data() + 7, nullptr, nullptr, false, icp_mode));
+    const int grid = std::max(1, std::min(div_up(n, ICP_BLOCK), c->sm_count * 4));   // depends on n only: the fold order is the same for every guess
+    LIMU_TRY(stage_in(c, c->tmp5, poses.data(), (size_t)(st.iterations + 1) * 7 * sizeof(double)));
+    LIMU_TRY(c->tmp2.reserve((size_t)grid * 2 * sizeof(double), c->stream));
+    if (icp_mode & LIMU_ICP_NN27)
+        k_icp_fitness<true><<<grid, ICP_BLOCK, 0, c->stream>>>(m->view(), c->in0.as<double>(), n, c->tmp5.as<double>(), st.iterations + 1, tau * tau, c->tmp2.as<double>());
+    else
+        k_icp_fitness<false><<<grid, ICP_BLOCK, 0, c->stream>>>(m->view(), c->in0.as<double>(), n, c->tmp5.as<double>(), st.iterations + 1, tau * tau, c->tmp2.as<double>());
+    LIMU_LAUNCHED();
+    std::vector<double> rows((size_t)grid * 2);
+    LIMU_CUDA_TRY(cudaMemcpyAsync(rows.data(), c->tmp2.p, rows.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    LIMU_TRY(check_status(c));
+    double inl = 0.0, d2 = 0.0;
+    for (int b = 0; b < grid; ++b) { inl += rows[2 * b]; d2 += rows[2 * b + 1]; }
+    res[7] = st.iterations; res[8] = st.converged; res[9] = inl; res[10] = d2;
+    return LIMU_OK;
+}
+
 extern "C" {
+
+int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init_guesses, int32_t k, double max_corresp_dist, double kernel,
+                   int icp_max_iteration, double est_threshold, int32_t icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best) {
+    LIMU_REQUIRE(m && n >= 0 && (n == 0 || xyz) && k >= 0 && (k == 0 || (init_guesses && poses_out)), "limu_icp_multi: bad arguments");
+    LIMU_REQUIRE((icp_mode & ~(LIMU_ICP_NN27 | LIMU_ICP_PLANE)) == 0, "limu_icp_multi: unknown icp_mode bits");
+    LIMU_REQUIRE(!(icp_mode & LIMU_ICP_PLANE), "limu_icp_multi: the point-to-plane variant is not available in the multi-hypothesis loop");
+    if (best) *best = -1;
+    if (k == 0) return LIMU_OK;
+    LIMU_TRY(bind(m->ctx));
+    LIMU_TRY(stage_in(m->ctx, m->ctx->in0, xyz, (size_t)n * 24));
+    std::vector<double> res((size_t)k * MULTI_OUT);
+    if (n <= 16384 && m->cap <= 64) {   // the latency shape, as icp_device would choose it for one hypothesis
+        LIMU_TRY(icp_multi_grouped(m, n, init_guesses, k, max_corresp_dist, kernel, icp_max_iteration, est_threshold, (icp_mode & LIMU_ICP_NN27) != 0, res.data()));
+    } else {
+        for (int h = 0; h < k; ++h)
+            LIMU_TRY(icp_multi_single(m, n, init_guesses + 7 * (size_t)h, max_corresp_dist, kernel, icp_max_iteration, est_threshold, icp_mode,
+                                      res.data() + (size_t)h * MULTI_OUT));
+    }
+    for (int h = 0; h < k; ++h) {   // best: most inliers, then the smaller rms, then the lower index
+        const double *r = res.data() + (size_t)h * MULTI_OUT;
+        const int64_t inl = (int64_t)r[9];
+        const double rms = inl > 0 ? sqrt(r[10] / (double)inl) : 0.0;
+        std::copy(r, r + 7, poses_out + 7 * (size_t)h);
+        if (out) { out[h].iterations = (int32_t)r[7]; out[h].converged = (int32_t)r[8]; out[h].inliers = inl; out[h].rms = rms; }
+        if (best) {
+            const double *b = *best >= 0 ? res.data() + (size_t)*best * MULTI_OUT : nullptr;
+            const int64_t binl = b ? (int64_t)b[9] : -1;
+            const double brms = b && binl > 0 ? sqrt(b[10] / (double)binl) : 0.0;
+            if (!b || inl > binl || (inl == binl && rms < brms)) *best = h;
+        }
+    }
+    return LIMU_OK;
+}
 
 int limu_icp(limu_map *m, const double *xyz, int64_t n, const double init_guess[7], double max_corresp_dist, double kernel, int icp_max_iteration,
              double est_threshold, double pose_out[7], limu_icp_stats *stats, double *est_trace, int64_t *ncorr_trace, double *hg_trace) {
