@@ -191,6 +191,41 @@ typedef struct limu_icp_hypothesis {
 } limu_icp_hypothesis;
 int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init_guesses, int32_t k, double max_corresp_dist, double kernel,
                    int icp_max_iteration, double est_threshold, int32_t icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best);
+/* Fitness of one scan at k given poses, with no Gauss-Newton loop (no counterpart in the reference): for pose p, the points moved by p, then
+ * the correspondence test of limu_icp_multi's fitness under icp_mode's neighbour rule: inliers[p] = #points whose match lies within
+ * max_corresp_dist, rms[p] = sqrt(sum d^2 / inliers) (0 without inliers). Nothing found -> (0,0,0), range-tested like a real point, as in
+ * the loop. A pose's score is the fitness limu_icp_multi reports for a hypothesis that ran 0 iterations from it: inliers equal, rms equal up
+ * to the order of the sum of d^2, which here depends on n only -- a pose's result is bit-identical whatever k is and wherever the pose sits in
+ * the list, and a non-finite or far-away pose affects only its own entry. poses: 7 k doubles; inliers / rms: k entries.
+ * icp_mode: LIMU_ICP_REFERENCE or LIMU_ICP_NN27 (LIMU_ICP_PLANE: LIMU_ERR_INVALID). Any max_points_per_voxel. Only reads the map (on a map
+ * of an odometry handle the call is ordered like limu_icp). */
+int limu_map_score_poses(limu_map *m, const double *xyz, int64_t n, const double *poses, int64_t k, double max_corresp_dist,
+                         int32_t icp_mode, int64_t *inliers, double *rms);
+/* Global relocalization without a coarse pose (no counterpart in the reference): a planar search grid in the frame of `center` (z, roll
+ * and pitch come from center, e.g. gravity from the IMU): candidate (i, j, l), index (l * ny + j) * nx + i, is center * D with
+ * D = {q = (0, 0, sin(t/2), cos(t/2)), t = (x_i, y_j, 0)}, x_i = (i - (nx-1)/2) * step_xy, y_j likewise, t = (l - (nyaw-1)/2) * step_yaw.
+ * nx, ny, nyaw >= 1; steps > 0. */
+typedef struct limu_reloc_grid {
+    double center[7];
+    int32_t nx, ny, nyaw, reserved0;
+    double step_xy, step_yaw;
+} limu_reloc_grid;
+typedef struct limu_reloc_candidate {
+    int64_t index;                    /* grid index */
+    double coarse_pose[7];            /* the candidate pose the score refers to */
+    int64_t coarse_inliers;
+    double coarse_rms;
+    double pose[7];                   /* after ICP from coarse_pose */
+    limu_icp_hypothesis icp;          /* iterations, converged, inliers, rms after the loop */
+} limu_reloc_candidate;
+/* Scores every candidate of the grid on the device (limu_map_score_poses' rule; candidate poses and scores never leave the device), keeps
+ * the n_refine best by (coarse inliers desc, coarse rms asc, index asc) -- an exact, deterministic selection, 1 <= n_refine <= 4096 --,
+ * runs limu_icp_multi from their coarse poses and returns them in that order in out[0 .. *n_out) (*n_out = min(n_refine, candidates));
+ * best = limu_icp_multi's rule over the refined results. The refined results are those limu_icp_multi returns from the same coarse poses,
+ * bit for bit. Device scratch grows with the grid: 16 bytes per candidate (LIMU_ERR_NOMEM when that does not fit). icp_mode as above. */
+int limu_relocalize(limu_map *m, const double *xyz, int64_t n, const limu_reloc_grid *grid, int32_t n_refine, double max_corresp_dist,
+                    double kernel, int icp_max_iteration, double est_threshold, int32_t icp_mode, limu_reloc_candidate *out,
+                    int32_t *n_out, int32_t *best);
 /* get_closest_neighbour under a neighbour rule (icp_mode as above); outputs as limu_map_closest. */
 int limu_map_closest_ex(limu_map *m, const double *xyz, int64_t n, int32_t icp_mode, double *out_xyz, int32_t *out_key, int32_t *out_rank);
 

@@ -59,5 +59,36 @@ namespace lidar
         r.best = best;
         return r;
     }
+
+    // Global relocalization without a coarse pose (limu_relocalize; no counterpart in the reference): every candidate of the planar grid
+    // of nx x ny x nyaw poses around `center` (x, y steps step_xy, yaw steps step_yaw; z, roll and pitch from center) is scored on the
+    // device, the n_refine best (most inliers, then the smaller rms, then the lower grid index) are refined by ICP_multi and returned in that
+    // order: candidates[i] holds the grid index, the coarse pose and score, and the refined pose and record; poses[i] is the refined pose.
+    // best: ICP_multi's rule over the refined results.
+    struct RelocalizeResult
+    {
+        std::vector<limu_reloc_candidate> candidates;
+        std::vector<SE3d> poses;
+        int best = -1;
+    };
+    inline RelocalizeResult relocalize(VoxelHashMap &local_map, const utils::Vec3dVector &points, const SE3d &center, const int nx, const int ny,
+                                       const int nyaw, const double step_xy, const double step_yaw, const int n_refine, const double max_corresp_dist,
+                                       const double kernel, const int &icp_max_iteration, const double &est_threshold)
+    {
+        limu_reloc_grid grid{};
+        limu_dropin::to_pose7(center, grid.center);
+        grid.nx = nx; grid.ny = ny; grid.nyaw = nyaw; grid.step_xy = step_xy; grid.step_yaw = step_yaw;
+        RelocalizeResult r;
+        r.candidates.resize(static_cast<size_t>(n_refine > 0 && n_refine <= 4096 ? n_refine : 1));
+        int32_t n_out = 0, best = -1;
+        limu_dropin::check(limu_relocalize(local_map.handle(), points.empty() ? nullptr : points.front().data(), static_cast<int64_t>(points.size()),
+                                           &grid, n_refine, max_corresp_dist, kernel, icp_max_iteration, est_threshold, LIMU_ICP_REFERENCE,
+                                           r.candidates.data(), &n_out, &best), "relocalize");
+        r.candidates.resize(static_cast<size_t>(n_out));
+        r.poses.reserve(r.candidates.size());
+        for (const limu_reloc_candidate &c : r.candidates) r.poses.push_back(limu_dropin::from_pose7(c.pose));
+        r.best = best;
+        return r;
+    }
 }
 #endif

@@ -45,6 +45,16 @@ class IcpHypothesis(C.Structure):
     _fields_ = [("iterations", C.c_int32), ("converged", C.c_int32), ("inliers", C.c_int64), ("rms", C.c_double)]
 
 
+class RelocGrid(C.Structure):
+    _fields_ = [("center", C.c_double * 7), ("nx", C.c_int32), ("ny", C.c_int32), ("nyaw", C.c_int32), ("reserved0", C.c_int32),
+                ("step_xy", C.c_double), ("step_yaw", C.c_double)]
+
+
+class RelocCandidate(C.Structure):
+    _fields_ = [("index", C.c_int64), ("coarse_pose", C.c_double * 7), ("coarse_inliers", C.c_int64), ("coarse_rms", C.c_double),
+                ("pose", C.c_double * 7), ("icp", IcpHypothesis)]
+
+
 class OdomConfig(C.Structure):
     _fields_ = [("voxel_size", C.c_double), ("max_range", C.c_double), ("max_points_per_voxel", C.c_int32),
                 ("deskew", C.c_int32), ("min_motion_th", C.c_double), ("icp_max_iteration", C.c_int32),
@@ -178,6 +188,9 @@ def lib():
             "limu_icp_ex": [_vp, _dp, C.c_int64, _dp, C.c_double, C.c_double, C.c_int, C.c_double, C.c_int32, _dp, C.POINTER(IcpStats), _dp, _lp, _dp],
             "limu_icp_multi": [_vp, _dp, C.c_int64, _dp, C.c_int32, C.c_double, C.c_double, C.c_int, C.c_double, C.c_int32, _dp, C.POINTER(IcpHypothesis),
                                C.POINTER(C.c_int32)],
+            "limu_map_score_poses": [_vp, _dp, C.c_int64, _dp, C.c_int64, C.c_double, C.c_int32, _lp, _dp],
+            "limu_relocalize": [_vp, _dp, C.c_int64, C.POINTER(RelocGrid), C.c_int32, C.c_double, C.c_double, C.c_int, C.c_double, C.c_int32,
+                                C.POINTER(RelocCandidate), C.POINTER(C.c_int32), C.POINTER(C.c_int32)],
             "limu_map_closest_ex": [_vp, _dp, C.c_int64, C.c_int32, _dp, _ip, _ip],
             "limu_icp_dev": [_vp, _vp, C.c_int64, _dp, C.c_double, C.c_double, C.c_int, C.c_double, _dp, C.POINTER(IcpStats)],
             "limu_comm_create": [_vp, C.c_int, C.c_int, C.c_char_p], "limu_comm_connect": [_vp, C.c_char_p], "limu_comm_destroy": [_vp],
@@ -571,6 +584,37 @@ class VoxelHashMap:
                 "converged": np.array([bool(hyp[i].converged) for i in range(k)], bool),
                 "inliers": np.array([hyp[i].inliers for i in range(k)], np.int64), "rms": np.array([hyp[i].rms for i in range(k)]),
                 "best": best.value}
+
+    def score_poses(self, xyz, poses, max_corresp_dist, icp_mode=0):
+        """Fitness of xyz at every row of poses [k, 7] without a Gauss-Newton loop (limu_map_score_poses): what icp_multi reports for a
+        hypothesis run for 0 iterations. Returns dict(inliers [k], rms [k])."""
+        xyz = _pts(xyz)
+        p = np.ascontiguousarray(np.asarray(poses, np.float64).reshape(-1, 7))
+        k = len(p)
+        inl, rms = np.zeros(max(k, 1), np.int64), np.zeros(max(k, 1))
+        _chk(lib().limu_map_score_poses(self.h, _d(xyz), len(xyz), _d(p), k, float(max_corresp_dist), int(icp_mode),
+                                        inl.ctypes.data_as(_lp), _d(rms)))
+        return {"inliers": inl[:k].copy(), "rms": rms[:k].copy()}
+
+    def relocalize(self, xyz, center, nx, ny, nyaw, step_xy, step_yaw, n_refine, max_corresp_dist, kernel, icp_max_iteration, est_threshold,
+                   icp_mode=0):
+        """Global relocalization (limu_relocalize): score the planar grid of nx x ny x nyaw candidates around center (index (l * ny + j) * nx + i),
+        keep the n_refine best by (inliers desc, rms asc, index asc) and run icp_multi from them. Returns dict of arrays in that order --
+        index, coarse_poses, coarse_inliers, coarse_rms, poses, iters, converged, inliers, rms -- and best (icp_multi's rule)."""
+        xyz = _pts(xyz)
+        g = RelocGrid()
+        g.center[:] = [float(v) for v in _pose(center)]
+        g.nx, g.ny, g.nyaw, g.step_xy, g.step_yaw = int(nx), int(ny), int(nyaw), float(step_xy), float(step_yaw)
+        cand = (RelocCandidate * max(1, min(int(n_refine), 4096)))()
+        n_out, best = C.c_int32(0), C.c_int32(-1)
+        _chk(lib().limu_relocalize(self.h, _d(xyz), len(xyz), C.byref(g), int(n_refine), float(max_corresp_dist), float(kernel),
+                                   int(icp_max_iteration), float(est_threshold), int(icp_mode), cand, C.byref(n_out), C.byref(best)))
+        c = cand[:n_out.value]
+        return {"index": np.array([x.index for x in c], np.int64), "coarse_poses": np.array([list(x.coarse_pose) for x in c]).reshape(-1, 7),
+                "coarse_inliers": np.array([x.coarse_inliers for x in c], np.int64), "coarse_rms": np.array([x.coarse_rms for x in c]),
+                "poses": np.array([list(x.pose) for x in c]).reshape(-1, 7), "iters": np.array([x.icp.iterations for x in c], np.int32),
+                "converged": np.array([bool(x.icp.converged) for x in c], bool), "inliers": np.array([x.icp.inliers for x in c], np.int64),
+                "rms": np.array([x.icp.rms for x in c]), "best": best.value}
 
     def icp_dev(self, xyz_dev_ptr, n, init_guess, max_corresp_dist, kernel, icp_max_iteration, est_threshold):
         pose = np.empty(7)

@@ -1359,6 +1359,110 @@ static __global__ void __launch_bounds__(ICP_BLOCK) k_icp_fitness(const MapView 
     }
 }
 
+// ---- pose scoring and global relocalization: the fitness of k_icp_multi at millions of poses, without a Gauss-Newton loop --------------
+// Where the poses come from: a list (7 doubles each), or the planar grid of limu_relocalize -- candidate p = (l * ny + j) * nx + i is
+// center * {q = (0, 0, sin(t_l / 2), cos(t_l / 2)), t = (x_i, y_j, 0)}, built where it is scored, so a grid never exists in memory.
+struct PoseSource {
+    const double *list;   // k x 7, or null: the grid
+    double center[7];
+    const double *yaw;    // nyaw x 2: sin(t_l / 2), cos(t_l / 2) (host libm: the table is tiny)
+    int64_t nx, ny;
+    double step_xy;
+    __device__ __forceinline__ Pose at(int64_t p) const {
+        if (list) return pose_load(list + 7 * p);
+        const int64_t i = p % nx, r = p / nx, j = r % ny, l = r / ny;
+        const double x = ((double)i - 0.5 * (double)(nx - 1)) * step_xy, y = ((double)j - 0.5 * (double)(ny - 1)) * step_xy;
+        return mul(pose_load(center), Pose{0.0, 0.0, yaw[2 * l], yaw[2 * l + 1], x, y, 0.0});
+    }
+};
+
+constexpr int SCORE_BLOCK = 256;
+
+// One warp per pose (a persistent grid of warps takes poses p, p + warps, ...), one lane per query: the points moved by the pose, the
+// correspondence test of k_icp_multi's fitness under the loop's neighbour rule (map_locate + block_closest / map_closest27, any cap), and a
+// per-pose reduction inside the warp -- so a pose's sums depend on n only, never on k, on the pose's place in the list or on the grid.
+// (Eight lanes per query, as in fitness_pass_grouped, was measured slower overall: DESIGN.md section 9.)
+// hist (optional): histogram of the inlier counts (n + 1 bins) for the selection of limu_relocalize.
+template <bool NN27>
+static __global__ void __launch_bounds__(SCORE_BLOCK) k_score_poses(const MapView map, const double *points, int64_t n, const PoseSource src,
+                                                                    int64_t k, double tau_sq, int64_t *inliers_out, double *rms_out,
+                                                                    unsigned long long *hist) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (SCORE_BLOCK / 32);
+    for (int64_t p = (int64_t)blockIdx.x * (SCORE_BLOCK / 32) + (threadIdx.x >> 5); p < k; p += warps) {   // warp-uniform
+        const Pose P = src.at(p);
+        long long inl = 0;
+        double d2sum = 0.0;
+        for (int64_t q = lane; q < n; q += 32) {
+            const V3 s = apply(P, V3{points[3 * q], points[3 * q + 1], points[3 * q + 2]});
+            Nearest nn;
+            nn.rank = -1;
+            if (NN27) {
+                nn = map_closest27(map, s);
+            } else {
+                int count = 0, own = 1;
+                const int slot = map_locate(map, s, &count, &own);
+                if (slot >= 0) block_closest(map, slot, count, s, nn);
+            }
+            const double d2 = nn.rank >= 0 ? sqnorm3(nn.x - s.x, nn.y - s.y, nn.z - s.z) : sqnorm3(s.x, s.y, s.z);   // nothing found -> (0,0,0)
+            if (d2 < tau_sq) { ++inl; d2sum += d2; }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) inl += __shfl_down_sync(0xFFFFFFFFu, inl, o);
+        d2sum = warp_sum(d2sum);
+        if (lane == 0) {
+            inliers_out[p] = inl;
+            rms_out[p] = inl > 0 ? sqrt(d2sum / (double)inl) : 0.0;   // limu_icp_multi's expression
+            if (hist) atomicAdd(hist + inl, 1ull);
+        }
+    }
+}
+
+// Exact top-M of limu_relocalize by (inliers desc, rms asc, index asc). The inlier histogram gives the class T the M-th candidate falls in;
+// inside that class the order is that of the 128-bit key (rms bits, index) -- rms >= 0, so its bits order like the values -- and a radix
+// select fixes that key's top `digits` bytes, eight bits per pass over the candidates: a candidate of class T is taken when its key's top
+// bytes are <= the prefix found (Sel::mh / ml mask them).
+struct Sel {
+    int64_t T;
+    unsigned long long mh, ml, ph, pl;
+};
+__device__ __forceinline__ bool sel_taken(const Sel &S, int64_t inl, double rms, int64_t p) {
+    if (inl != S.T) return inl > S.T;
+    const unsigned long long h = (unsigned long long)__double_as_longlong(rms) & S.mh, l = (unsigned long long)p & S.ml;
+    return h < S.ph || (h == S.ph && l <= S.pl);
+}
+// Histogram of key byte `digit` (0: the top byte of the rms bits ... 15: the low byte of the index) over the class-T candidates whose
+// decided bytes equal the prefix.
+static __global__ void __launch_bounds__(256) k_select_digit(const int64_t *inliers, const double *rms, int64_t k, const Sel S, int digit,
+                                                             unsigned long long *hist256) {
+    __shared__ unsigned int h[256];
+    h[threadIdx.x] = 0u;
+    __syncthreads();
+    for (int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x; p < k; p += (int64_t)gridDim.x * 256) {
+        if (inliers[p] != S.T) continue;
+        const unsigned long long hi = (unsigned long long)__double_as_longlong(rms[p]), lo = (unsigned long long)p;
+        if ((hi & S.mh) != S.ph || (lo & S.ml) != S.pl) continue;
+        const unsigned int d = (unsigned int)((digit < 8 ? hi >> (56 - 8 * digit) : lo >> (56 - 8 * (digit - 8))) & 255u);
+        atomicAdd(&h[d], 1u);
+    }
+    __syncthreads();
+    if (h[threadIdx.x]) atomicAdd(hist256 + threadIdx.x, (unsigned long long)h[threadIdx.x]);
+}
+// The selected candidates as (index, inliers, rms bits), in no particular order (the host sorts at most 4096 of them).
+static __global__ void __launch_bounds__(256) k_select_gather(const int64_t *inliers, const double *rms, int64_t k, const Sel S,
+                                                              unsigned long long *count, int64_t cap, long long *rec) {
+    for (int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x; p < k; p += (int64_t)gridDim.x * 256) {
+        if (!sel_taken(S, inliers[p], rms[p], p)) continue;
+        const unsigned long long at = atomicAdd(count, 1ull);
+        if ((int64_t)at < cap) { rec[3 * at] = p; rec[3 * at + 1] = inliers[p]; rec[3 * at + 2] = __double_as_longlong(rms[p]); }
+    }
+}
+// The poses of m grid candidates, by index.
+static __global__ void k_grid_poses(const PoseSource src, const int64_t *index, int m, double *poses) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < m) pose_store(src.at(index[i]), poses + 7 * (size_t)i);
+}
+
 #ifdef LIMU_ICP_PHASE_TIMING
 extern "C" int limu_debug_frame_marks(double out[72]) {
     unsigned long long h[72];
@@ -1509,7 +1613,7 @@ static int icp_common(limu_map *m, const double *points_dev, int64_t n, const do
     return check_status(c);
 }
 
-// All k hypotheses of the latency shape in one cooperative launch; res: k x MULTI_OUT doubles (host).
+// All k hypotheses of the latency shape in one cooperative launch; guesses: k x 7 doubles (device); res: k x MULTI_OUT doubles (host).
 static int icp_multi_grouped(limu_map *m, int64_t n, const double *guesses, int k, double tau, double th, int max_iter, double eps, bool nn27, double *res) {
     limu_ctx *c = m->ctx;
     const int G = icp_multi_group_ctas(n);
@@ -1522,7 +1626,6 @@ static int icp_multi_grouped(limu_map *m, int64_t n, const double *guesses, int 
     const int groups = std::max(1, std::min(k, resident / G));
     LIMU_TRY(c->tmp4.reserve((size_t)groups * (size_t)std::max<int64_t>(n, 1) * 24, c->stream));   // one working cloud per running group
     LIMU_TRY(icp_partials_reserve(c, c->ll_rows, c->stream));
-    LIMU_TRY(stage_in(c, c->tmp5, guesses, (size_t)k * 7 * sizeof(double)));
     LIMU_TRY(c->tmp3.reserve((size_t)k * MULTI_OUT * sizeof(double), c->stream));
     MultiArgs M;
     memset(&M, 0, sizeof M);
@@ -1534,7 +1637,7 @@ static int icp_multi_grouped(limu_map *m, int64_t n, const double *guesses, int 
     A.ll_stamp_base = c->ll_seq;
     const unsigned int waves = (unsigned int)div_up(k, groups);   // a group makes at most max_iter + 1 exchanges per hypothesis (the last: its fitness)
     c->ll_seq = (c->ll_seq + waves * ((unsigned int)std::max(max_iter, 0) + 1u) + 2u) & 0x7FFFFFFFu;
-    M.guesses = c->tmp5.as<double>(); M.out = c->tmp3.as<double>(); M.k = k; M.group_ctas = G;
+    M.guesses = guesses; M.out = c->tmp3.as<double>(); M.k = k; M.group_ctas = G;
     void *args[] = {&M};
     LIMU_CUDA_TRY(cudaLaunchCooperativeKernel(fn, dim3(groups * G), dim3(ICP_BLOCK), args, 0, c->stream));
     LIMU_LAUNCHED();
@@ -1566,24 +1669,20 @@ static int icp_multi_single(limu_map *m, int64_t n, const double guess[7], doubl
     return LIMU_OK;
 }
 
-extern "C" {
-
-int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init_guesses, int32_t k, double max_corresp_dist, double kernel,
-                   int icp_max_iteration, double est_threshold, int32_t icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best) {
-    LIMU_REQUIRE(m && n >= 0 && (n == 0 || xyz) && k >= 0 && (k == 0 || (init_guesses && poses_out)), "limu_icp_multi: bad arguments");
-    LIMU_REQUIRE((icp_mode & ~(LIMU_ICP_NN27 | LIMU_ICP_PLANE)) == 0, "limu_icp_multi: unknown icp_mode bits");
-    LIMU_REQUIRE(!(icp_mode & LIMU_ICP_PLANE), "limu_icp_multi: the point-to-plane variant is not available in the multi-hypothesis loop");
-    if (best) *best = -1;
-    if (k == 0) return LIMU_OK;
-    LIMU_TRY(bind(m->ctx));
-    LIMU_TRY(stage_in(m->ctx, m->ctx->in0, xyz, (size_t)n * 24));
+// limu_icp_multi on the scan in c->in0 from k guesses, given on the host and optionally already on the device (guesses_dev).
+static int icp_multi_run(limu_map *m, int64_t n, const double *guesses, const double *guesses_dev, int k, double tau, double th, int max_iter,
+                         double eps, int icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best) {
+    limu_ctx *c = m->ctx;
     std::vector<double> res((size_t)k * MULTI_OUT);
     if (n <= 16384 && m->cap <= 64) {   // the latency shape, as icp_device would choose it for one hypothesis
-        LIMU_TRY(icp_multi_grouped(m, n, init_guesses, k, max_corresp_dist, kernel, icp_max_iteration, est_threshold, (icp_mode & LIMU_ICP_NN27) != 0, res.data()));
+        if (!guesses_dev) {
+            LIMU_TRY(stage_in(c, c->tmp5, guesses, (size_t)k * 7 * sizeof(double)));
+            guesses_dev = c->tmp5.as<double>();
+        }
+        LIMU_TRY(icp_multi_grouped(m, n, guesses_dev, k, tau, th, max_iter, eps, (icp_mode & LIMU_ICP_NN27) != 0, res.data()));
     } else {
         for (int h = 0; h < k; ++h)
-            LIMU_TRY(icp_multi_single(m, n, init_guesses + 7 * (size_t)h, max_corresp_dist, kernel, icp_max_iteration, est_threshold, icp_mode,
-                                      res.data() + (size_t)h * MULTI_OUT));
+            LIMU_TRY(icp_multi_single(m, n, guesses + 7 * (size_t)h, tau, th, max_iter, eps, icp_mode, res.data() + (size_t)h * MULTI_OUT));
     }
     for (int h = 0; h < k; ++h) {   // best: most inliers, then the smaller rms, then the lower index
         const double *r = res.data() + (size_t)h * MULTI_OUT;
@@ -1598,6 +1697,193 @@ int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init
             if (!b || inl > binl || (inl == binl && rms < brms)) *best = h;
         }
     }
+    return LIMU_OK;
+}
+
+// Scores k poses of `src` against the scan in c->in0: inliers into c->tmp0, rms into c->tmp1 (k each); hist: see k_score_poses.
+static int score_poses_device(limu_map *m, int64_t n, const PoseSource &src, int64_t k, double tau, bool nn27, unsigned long long *hist) {
+    limu_ctx *c = m->ctx;
+    LIMU_TRY(c->tmp0.reserve((size_t)k * sizeof(int64_t), c->stream));
+    LIMU_TRY(c->tmp1.reserve((size_t)k * sizeof(double), c->stream));
+    const void *fn = nn27 ? (const void *)k_score_poses<true> : (const void *)k_score_poses<false>;
+    int per_sm = 0;
+    LIMU_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, SCORE_BLOCK, 0));
+    const int64_t blocks = std::max<int64_t>(1, std::min<int64_t>((k + SCORE_BLOCK / 32 - 1) / (SCORE_BLOCK / 32), (int64_t)std::max(per_sm, 1) * c->sm_count));
+    const MapView view = m->view();
+    const double *points = c->in0.as<double>();
+    const double tau_sq = tau * tau;
+    int64_t *inl = c->tmp0.as<int64_t>();
+    double *rms = c->tmp1.as<double>();
+    void *args[] = {(void *)&view, (void *)&points, (void *)&n, (void *)&src, (void *)&k, (void *)&tau_sq, (void *)&inl, (void *)&rms, (void *)&hist};
+    LIMU_CUDA_TRY(cudaLaunchKernel(fn, dim3((unsigned int)blocks), dim3(SCORE_BLOCK), args, 0, c->stream));
+    LIMU_LAUNCHED();
+    return LIMU_OK;
+}
+
+// Size of the allocation DevBuf::reserve would make for `want` bytes (0: none).
+static size_t reserve_growth(const DevBuf &b, size_t want) {
+    if (want <= b.bytes) return 0;
+    size_t nb = b.bytes ? b.bytes : 256;
+    while (nb < want) {
+        if (nb > SIZE_MAX / 2) return SIZE_MAX;
+        nb *= 2;
+    }
+    return nb;
+}
+
+// limu_relocalize's candidate scores for a grid of k candidates: LIMU_ERR_NOMEM when they do not fit the device.
+static int reserve_scores(limu_ctx *c, int64_t k) {
+    size_t fr = 0, total = 0;
+    LIMU_CUDA_TRY(cudaMemGetInfo(&fr, &total));
+    const bool fits = (uint64_t)k <= SIZE_MAX / 8 && [&] {
+        const size_t a = reserve_growth(c->tmp0, (size_t)k * 8), b = reserve_growth(c->tmp1, (size_t)k * 8);
+        // (reserve allocates before it frees: tmp0's new block, then tmp1's with tmp0's old block back)
+        return a <= fr && b <= fr - a + (a ? c->tmp0.bytes : 0);
+    }();
+    if (!fits) { set_error("limu_relocalize: the scores of %lld candidates (16 bytes each) do not fit in device memory", (long long)k); return LIMU_ERR_NOMEM; }
+    LIMU_TRY(c->tmp0.reserve((size_t)k * 8, c->stream));
+    return c->tmp1.reserve((size_t)k * 8, c->stream);
+}
+
+extern "C" {
+
+int limu_icp_multi(limu_map *m, const double *xyz, int64_t n, const double *init_guesses, int32_t k, double max_corresp_dist, double kernel,
+                   int icp_max_iteration, double est_threshold, int32_t icp_mode, double *poses_out, limu_icp_hypothesis *out, int32_t *best) {
+    LIMU_REQUIRE(m && n >= 0 && (n == 0 || xyz) && k >= 0 && (k == 0 || (init_guesses && poses_out)), "limu_icp_multi: bad arguments");
+    LIMU_REQUIRE((icp_mode & ~(LIMU_ICP_NN27 | LIMU_ICP_PLANE)) == 0, "limu_icp_multi: unknown icp_mode bits");
+    LIMU_REQUIRE(!(icp_mode & LIMU_ICP_PLANE), "limu_icp_multi: the point-to-plane variant is not available in the multi-hypothesis loop");
+    if (best) *best = -1;
+    if (k == 0) return LIMU_OK;
+    LIMU_TRY(bind(m->ctx));
+    LIMU_TRY(stage_in(m->ctx, m->ctx->in0, xyz, (size_t)n * 24));
+    return icp_multi_run(m, n, init_guesses, nullptr, k, max_corresp_dist, kernel, icp_max_iteration, est_threshold, icp_mode, poses_out, out, best);
+}
+
+int limu_map_score_poses(limu_map *m, const double *xyz, int64_t n, const double *poses, int64_t k, double max_corresp_dist, int32_t icp_mode,
+                         int64_t *inliers, double *rms) {
+    LIMU_REQUIRE(m && n >= 0 && (n == 0 || xyz) && k >= 0 && (k == 0 || (poses && inliers && rms)), "limu_map_score_poses: bad arguments");
+    LIMU_REQUIRE((icp_mode & ~(LIMU_ICP_NN27 | LIMU_ICP_PLANE)) == 0, "limu_map_score_poses: unknown icp_mode bits");
+    LIMU_REQUIRE(!(icp_mode & LIMU_ICP_PLANE), "limu_map_score_poses: point-to-plane scoring is not available");
+    if (k == 0) return LIMU_OK;
+    limu_ctx *c = m->ctx;
+    LIMU_TRY(bind(c));
+    LIMU_TRY(stage_in(c, c->in0, xyz, (size_t)n * 24));
+    LIMU_TRY(stage_in(c, c->tmp5, poses, (size_t)k * 7 * sizeof(double)));
+    PoseSource src;
+    memset(&src, 0, sizeof src);
+    src.list = c->tmp5.as<double>();
+    LIMU_TRY(score_poses_device(m, n, src, k, max_corresp_dist, (icp_mode & LIMU_ICP_NN27) != 0, nullptr));
+    LIMU_CUDA_TRY(cudaMemcpyAsync(inliers, c->tmp0.p, (size_t)k * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+    LIMU_CUDA_TRY(cudaMemcpyAsync(rms, c->tmp1.p, (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    return check_status(c);
+}
+
+int limu_relocalize(limu_map *m, const double *xyz, int64_t n, const limu_reloc_grid *grid, int32_t n_refine, double max_corresp_dist, double kernel,
+                    int icp_max_iteration, double est_threshold, int32_t icp_mode, limu_reloc_candidate *out, int32_t *n_out, int32_t *best) {
+    LIMU_REQUIRE(m && grid && out && n >= 0 && (n == 0 || xyz), "limu_relocalize: bad arguments");
+    LIMU_REQUIRE((icp_mode & ~(LIMU_ICP_NN27 | LIMU_ICP_PLANE)) == 0, "limu_relocalize: unknown icp_mode bits");
+    LIMU_REQUIRE(!(icp_mode & LIMU_ICP_PLANE), "limu_relocalize: point-to-plane scoring is not available");
+    LIMU_REQUIRE(n_refine >= 1 && n_refine <= 4096, "limu_relocalize: n_refine must be in 1 ... 4096");
+    LIMU_REQUIRE(grid->nx >= 1 && grid->ny >= 1 && grid->nyaw >= 1, "limu_relocalize: every grid count must be >= 1");
+    LIMU_REQUIRE(grid->step_xy > 0.0 && grid->step_yaw > 0.0, "limu_relocalize: the grid steps must be > 0");
+    if (n_out) *n_out = 0;
+    if (best) *best = -1;
+    limu_ctx *c = m->ctx;
+    LIMU_TRY(bind(c));
+    const int64_t nxy = (int64_t)grid->nx * grid->ny;
+    if (nxy > INT64_MAX / grid->nyaw) { set_error("limu_relocalize: the grid has more than 2^63 candidates"); return LIMU_ERR_NOMEM; }
+    const int64_t K = nxy * grid->nyaw;
+    const int M = (int)std::min<int64_t>(n_refine, K);
+    LIMU_TRY(reserve_scores(c, K));
+    LIMU_TRY(stage_in(c, c->in0, xyz, (size_t)n * 24));
+    // out2: yaw table (2 nyaw doubles), then the selected indices in ranking order (M), then their coarse poses (7 M)
+    std::vector<double> yaw(2 * (size_t)grid->nyaw);
+    for (int l = 0; l < grid->nyaw; ++l) {
+        const double t = ((double)l - 0.5 * (double)(grid->nyaw - 1)) * grid->step_yaw;
+        yaw[2 * l] = sin(t / 2.0); yaw[2 * l + 1] = cos(t / 2.0);
+    }
+    LIMU_TRY(c->out2.reserve((yaw.size() + 8 * (size_t)M) * 8, c->stream));
+    LIMU_CUDA_TRY(cudaMemcpyAsync(c->out2.p, yaw.data(), yaw.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    int64_t *d_index = reinterpret_cast<int64_t *>(c->out2.as<double>() + yaw.size());
+    double *d_poses = c->out2.as<double>() + yaw.size() + M;
+    PoseSource src;
+    memset(&src, 0, sizeof src);
+    std::copy(grid->center, grid->center + 7, src.center);
+    src.yaw = c->out2.as<double>(); src.nx = grid->nx; src.ny = grid->ny; src.step_xy = grid->step_xy;
+    // out0: inlier histogram (n + 1), digit histogram (256), gather counter; out1: the gathered records (3 M)
+    LIMU_TRY(c->out0.reserve(((size_t)n + 1 + 256 + 1) * 8, c->stream));
+    LIMU_TRY(c->out1.reserve((size_t)M * 3 * 8, c->stream));
+    unsigned long long *hist = c->out0.as<unsigned long long>(), *hist256 = hist + n + 1, *count = hist256 + 256;
+    LIMU_CUDA_TRY(cudaMemsetAsync(hist, 0, ((size_t)n + 1) * 8, c->stream));
+    LIMU_TRY(score_poses_device(m, n, src, K, max_corresp_dist, (icp_mode & LIMU_ICP_NN27) != 0, hist));
+    std::vector<unsigned long long> h((size_t)n + 1);
+    LIMU_CUDA_TRY(cudaMemcpyAsync(h.data(), hist, h.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    LIMU_TRY(check_status(c));
+    // the class of the M-th candidate, and how many of it are taken
+    Sel S;
+    memset(&S, 0, sizeof S);
+    int64_t above = 0;
+    for (S.T = n; above + (int64_t)h[S.T] < M; --S.T) above += (int64_t)h[S.T];
+    uint64_t need = (uint64_t)(M - above);
+    const int sel_blocks = (int)std::max<int64_t>(1, std::min<int64_t>((K + 255) / 256, (int64_t)c->sm_count * 8));
+    if (need < h[S.T]) {
+        unsigned long long hd[256];
+        for (int digit = 0; digit < 16; ++digit) {
+            const int shift = digit < 8 ? 56 - 8 * digit : 56 - 8 * (digit - 8);
+            unsigned long long &mask = digit < 8 ? S.mh : S.ml, &prefix = digit < 8 ? S.ph : S.pl;
+            if (digit >= 8 && ((uint64_t)(K - 1) >> shift) == 0) { mask |= 0xFFull << shift; continue; }   // an index byte that is 0 for every candidate
+            LIMU_CUDA_TRY(cudaMemsetAsync(hist256, 0, 256 * 8, c->stream));
+            k_select_digit<<<sel_blocks, 256, 0, c->stream>>>(c->tmp0.as<int64_t>(), c->tmp1.as<double>(), K, S, digit, hist256);
+            LIMU_LAUNCHED();
+            LIMU_CUDA_TRY(cudaMemcpyAsync(hd, hist256, sizeof hd, cudaMemcpyDeviceToHost, c->stream));
+            LIMU_CUDA_TRY(cudaStreamSynchronize(c->stream));
+            int d = 0;
+            while (hd[d] < need) need -= hd[d++];   // (d < 256: the candidates left hold at least `need`)
+            mask |= 0xFFull << shift;
+            prefix |= (unsigned long long)d << shift;
+            if (hd[d] == need) break;   // every candidate of this byte value is taken
+        }
+    }
+    LIMU_CUDA_TRY(cudaMemsetAsync(count, 0, 8, c->stream));
+    k_select_gather<<<sel_blocks, 256, 0, c->stream>>>(c->tmp0.as<int64_t>(), c->tmp1.as<double>(), K, S, count, M, c->out1.as<long long>());
+    LIMU_LAUNCHED();
+    std::vector<long long> rec(3 * (size_t)M);
+    unsigned long long got = 0;
+    LIMU_CUDA_TRY(cudaMemcpyAsync(&got, count, 8, cudaMemcpyDeviceToHost, c->stream));
+    LIMU_CUDA_TRY(cudaMemcpyAsync(rec.data(), c->out1.p, rec.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    LIMU_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (got != (unsigned long long)M) { set_error("limu_relocalize: selected %llu candidates instead of %d", got, M); return LIMU_ERR_CUDA; }
+    std::vector<int> order(M);
+    for (int i = 0; i < M; ++i) order[i] = i;
+    std::sort(order.begin(), order.end(), [&](int a, int b) {   // inliers desc, rms asc (its bits order like the values), index asc
+        const long long *x = &rec[3 * (size_t)a], *y = &rec[3 * (size_t)b];
+        if (x[1] != y[1]) return x[1] > y[1];
+        if (x[2] != y[2]) return (unsigned long long)x[2] < (unsigned long long)y[2];
+        return x[0] < y[0];
+    });
+    std::vector<int64_t> index(M);
+    for (int i = 0; i < M; ++i) index[i] = rec[3 * (size_t)order[i]];
+    LIMU_CUDA_TRY(cudaMemcpyAsync(d_index, index.data(), (size_t)M * 8, cudaMemcpyHostToDevice, c->stream));
+    k_grid_poses<<<div_up(M, 128), 128, 0, c->stream>>>(src, d_index, M, d_poses);
+    LIMU_LAUNCHED();
+    std::vector<double> coarse(7 * (size_t)M), refined(7 * (size_t)M);
+    LIMU_CUDA_TRY(cudaMemcpyAsync(coarse.data(), d_poses, coarse.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    LIMU_TRY(check_status(c));
+    std::vector<limu_icp_hypothesis> hyp(M);
+    int32_t b = -1;
+    LIMU_TRY(icp_multi_run(m, n, coarse.data(), d_poses, M, max_corresp_dist, kernel, icp_max_iteration, est_threshold, icp_mode, refined.data(), hyp.data(), &b));
+    for (int i = 0; i < M; ++i) {
+        const long long *r = &rec[3 * (size_t)order[i]];
+        limu_reloc_candidate &o = out[i];
+        o.index = r[0];
+        std::copy(&coarse[7 * (size_t)i], &coarse[7 * (size_t)i] + 7, o.coarse_pose);
+        o.coarse_inliers = r[1];
+        memcpy(&o.coarse_rms, &r[2], 8);
+        std::copy(&refined[7 * (size_t)i], &refined[7 * (size_t)i] + 7, o.pose);
+        o.icp = hyp[i];
+    }
+    if (n_out) *n_out = M;
+    if (best) *best = b;
     return LIMU_OK;
 }
 
